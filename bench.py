@@ -35,6 +35,7 @@ ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 
 ALG_BYTES_PER_VOXEL = 16.0  # read v, read w, write v, write w (fp32) -- SURVEY 8d
+DUMP_VOXELS = 4_000_000     # --dump-outputs: voxels sampled per array (2 float32 arrays, <= 32 MB in all)
 
 
 def measured_peaks():
@@ -106,6 +107,17 @@ class ClockSampler:
         if sm:
             out = {"sm_mhz": float(np.median(sm)), "sm_max_mhz": float(max(mx)), "reasons": sorted(reasons), "samples": len(sm)}
         return out
+
+
+def dump_sample(n_voxels, dev):
+    """Voxel indices that --dump-outputs writes: every voxel of a volume up to DUMP_VOXELS, else a fixed seeded sample (sorted,
+    unique), so that two builds run with the same arguments dump the same voxels."""
+    import torch
+    if n_voxels <= DUMP_VOXELS:
+        idx = np.arange(n_voxels)
+    else:
+        idx = np.unique(np.random.default_rng(0).integers(0, n_voxels, DUMP_VOXELS))
+    return torch.from_numpy(idx).to(dev)
 
 
 def build_scene(res, n_nodes, k, n_views, seed=0):
@@ -246,6 +258,8 @@ def run_ours(args):
     if world != args.gpus:
         if world == 1 and args.gpus > 1:
             raise SystemExit("launch with torch.distributed.run for --gpus > 1")
+    if args.dump_outputs and world > 1:
+        raise SystemExit("--dump-outputs is implemented for one GPU")
     torch.cuda.set_device(local_rank)
     dev = torch.device("cuda", local_rank)
     if world > 1:
@@ -321,10 +335,17 @@ def run_ours(args):
         parity = parity_check(args, sc, st, partition["slabs"], comm, rank, world, dev)
         st.reset()
 
+    dump_idx = dump_sample(nvox_rank, dev) if args.dump_outputs else None
     sampler = ClockSampler(local_rank) if rank == 0 else None
     if sampler:
         sampler.start()
     ms_total = st.timed(st.step_resident, args.steps, args.warmup, depth_dev, barrier)
+    dumped = None
+    if dump_idx is not None:
+        # what a caller of the timed path receives: the (tsdf, weight) volume after the last timed step, gathered before any
+        # later (untimed) step changes it
+        dumped = {"tsdf": st.vol.tsdf.view(-1)[dump_idx], "weight": st.vol.weight.view(-1)[dump_idx]}
+        torch.cuda.synchronize()
     # the K timed steps last only a few tens of ms; keep the same step running (untimed, identical count on every rank so
     # that the collectives match) until the 20 ms sampler has seen ~0.4 s of this load
     n_extra = max(0, int(400.0 / max(ms_total / args.steps, 1e-3)) - args.steps)
@@ -468,6 +489,10 @@ def run_ours(args):
         leg("gn_depth_frame", lambda: bench_gn_depth_frame(args, dev, rank, world, comm))
     if rank == 0 and world == 1 and not args.no_cpu_baseline:
         out["cpu_baseline"] = cpu_baseline(sc, grid, budget_s=args.cpu_seconds)
+    if dumped is not None:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, t in dumped.items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), t.cpu().numpy())
     if rank == 0:
         print(json.dumps(out))
     if world > 1:
@@ -971,7 +996,12 @@ def main():
     ap.add_argument("--gn-iters", type=int, default=15)
     ap.add_argument("--cpu-seconds", type=float, default=12.0)
     ap.add_argument("--ref-sample", type=int, default=1_600_000)
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write the TSDF volume of the last timed step as DIR/tsdf.npy "
+                                                          "and DIR/weight.npy (float32; a fixed seeded sample of %d voxels of a larger "
+                                                          "volume, see dump_sample)" % DUMP_VOXELS)
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     if args.impl == "reference":
         run_reference(args)

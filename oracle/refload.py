@@ -1,8 +1,8 @@
 """Loader for the UNMODIFIED reference (nintendops/DynamicFusion_Body) -- test infrastructure only.
 
-The reference is pure Python and lives read-only at /root/reference in the authoring container; it
-does NOT exist on the GPU box.  This module is only used (a) by tests that are skipped when the
-reference is absent and (b) by tests/golden/make_golden.py, which executes the reference to
+The reference is pure Python and is not part of this repository: put a checkout of it at oracle/_ref/ (ignored by git)
+or name one with DFB_REFERENCE_ROOT.  This module is only used (a) by tests that are skipped when the
+reference is absent and (b) by tests/golden/make_golden*.py, which execute the reference to
 produce the committed golden fixtures.  Nothing in the product package imports it.
 
 `import core` pulls TensorFlow-1, PyOpenGL, scikit-image and pyopencl (core/__init__.py:1-5,
@@ -15,7 +15,7 @@ import os
 import sys
 import types
 
-REFERENCE_ROOT = os.environ.get("DFB_REFERENCE_ROOT", "/root/reference")
+REFERENCE_ROOT = os.environ.get("DFB_REFERENCE_ROOT", os.path.join(os.path.dirname(os.path.abspath(__file__)), "_ref"))
 
 
 def available() -> bool:

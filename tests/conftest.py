@@ -11,7 +11,7 @@ for p in (ROOT, os.path.join(ROOT, "tests")):
 
 def pytest_configure(config):
     config.addinivalue_line("markers", "gpu: needs a CUDA device (run on the B200 box with -m gpu)")
-    config.addinivalue_line("markers", "reference: executes the unmodified reference from /root/reference (skipped when absent)")
+    config.addinivalue_line("markers", "reference: executes the unmodified reference checkout at oracle/_ref/ (skipped when absent)")
 
 
 @pytest.fixture(scope="session")

@@ -1,5 +1,5 @@
-"""Generate tests/golden/reference_vectors.npz by EXECUTING THE UNMODIFIED REFERENCE (/root/reference) on small
-seeded inputs.  Run in the authoring container only:   python tests/golden/make_golden.py
+"""Generate tests/golden/reference_vectors.npz by EXECUTING THE UNMODIFIED REFERENCE (a checkout at oracle/_ref/,
+see oracle/refload.py) on small seeded inputs:   python tests/golden/make_golden.py
 
 The reference has no golden vectors of its own beyond three quaternion doctests (core/util.py:146-153,176-194,
 258-260); these fixtures pin the oracle (oracle/*.py) to the reference's actual behaviour for every hot-path

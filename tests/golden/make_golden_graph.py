@@ -1,6 +1,6 @@
-"""Generate tests/golden/reference_graph_vectors.npz by EXECUTING THE UNMODIFIED REFERENCE (/root/reference) for the
-SURVEY 8f rows next to the hot paths: closest-point correspondences (Fusion / FusionDM.setupCorrespondences),
-`uniform_sample`, and `Fusion.update_graph`.  Run in the authoring container only:
+"""Generate tests/golden/reference_graph_vectors.npz by EXECUTING THE UNMODIFIED REFERENCE (a checkout at oracle/_ref/,
+see oracle/refload.py) for the SURVEY 8f rows next to the hot paths: closest-point correspondences (Fusion /
+FusionDM.setupCorrespondences), `uniform_sample`, and `Fusion.update_graph`:
 
     python tests/golden/make_golden_graph.py
 

@@ -1,7 +1,7 @@
 """Re-encode the reference's only data asset, meshes/original.obj (canonical body mesh of frame 0,
 meshes/README:1), as a compact npz fixture for tests and benchmarks.
 
-Run in the authoring container (needs /root/reference):  python tests/golden/make_mesh_fixture.py
+Needs a reference checkout (oracle/_ref/ or $DFB_REFERENCE_ROOT):  python tests/golden/make_mesh_fixture.py
 OBJ parsing follows the reference's own loader semantics (core/meshutil.py:12-39: 'v' lines -> vertices,
 'f' lines -> first index of each a/b/c triple, 0-based if the minimum index is 0).
 """
@@ -10,8 +10,9 @@ import sys
 
 import numpy as np
 
-REF = os.environ.get("DFB_REFERENCE_ROOT", "/root/reference")
-OUT = os.path.join(os.path.dirname(os.path.abspath(__file__)), "body_mesh.npz")
+HERE = os.path.dirname(os.path.abspath(__file__))
+REF = os.environ.get("DFB_REFERENCE_ROOT", os.path.join(os.path.dirname(os.path.dirname(HERE)), "oracle", "_ref"))
+OUT = os.path.join(HERE, "body_mesh.npz")
 
 
 def main():

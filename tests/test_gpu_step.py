@@ -118,3 +118,38 @@ def test_comm_single_rank_and_step_with_prefetch():
     torch.cuda.synchronize()
     assert torch.equal(vol.tsdf, vol0.tsdf) and torch.equal(vol.weight, vol0.weight)
     comm.close(); comm2.close()
+
+
+def test_bench_dump_outputs_hold_the_last_timed_step(tmp_path):
+    """bench.py --dump-outputs writes the volume the timed path leaves after its last timed step: the same frames (warm-up +
+    timed) through plain update calls give the same voxels bit for bit, and the JSON line counts the requested timed steps."""
+    import json
+    import os
+    import subprocess
+    import sys
+    import torch
+    import bench
+    from dynamicfusion_body_b200 import engine
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    res, nodes, steps, warmup = 64, 200, 2, 3
+    out = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--gpus", "1", "--steps", str(steps), "--warmup", str(warmup),
+                          "--res", str(res), "--nodes", str(nodes), "--no-gn", "--no-configs", "--no-cpu-baseline", "--dump-outputs", str(tmp_path)],
+                         capture_output=True, text=True, timeout=900)
+    assert out.returncode == 0, out.stderr[-2000:]
+    assert json.loads([ln for ln in out.stdout.splitlines() if ln.startswith("{")][-1])["steps"] == steps
+    assert sorted(os.listdir(tmp_path)) == ["tsdf.npy", "weight.npy"]
+    tsdf, weight = np.load(tmp_path / "tsdf.npy"), np.load(tmp_path / "weight.npy")
+    assert tsdf.dtype == weight.dtype == np.float32 and tsdf.shape == weight.shape == (res ** 3,)
+    sc = bench.build_scene(res, nodes, 4, 1)
+    dqs = bench.frame_dqs(sc, 15)
+    dev = torch.device("cuda", 0)
+    wf = engine.DeviceWarpField(4, dev)
+    wf.set_nodes(sc.node_pos, sc.node_dq, np.float32(sc.node_w))
+    vol = engine.DeviceVolume((res, res, res), device=dev, fill=sc.tdist)
+    depth = torch.from_numpy(sc.depths).to(dev)
+    for i in range(warmup + steps):
+        wf.set_dq(torch.from_numpy(dqs[i % len(dqs)]).to(dev))
+        engine.update_projective(vol, wf, sc.lw, depth, sc.K, sc.Kinv, sc.extrinsics, sc.tdist)
+    torch.cuda.synchronize()
+    assert (weight > 0).any()
+    assert np.array_equal(weight, vol.weight.cpu().numpy().ravel()) and np.array_equal(tsdf, vol.tsdf.cpu().numpy().ravel())

@@ -1,5 +1,5 @@
-"""Oracle against the UNMODIFIED reference executed live from /root/reference (skipped where it is absent, e.g. on
-the GPU box -- the committed golden vectors cover that case).  Randomised inputs beyond the golden set."""
+"""Oracle against the UNMODIFIED reference executed live from a checkout at oracle/_ref/ (see oracle/refload.py; skipped
+where it is absent -- the committed golden vectors cover that case).  Randomised inputs beyond the golden set."""
 import numpy as np
 import pytest
 
@@ -8,7 +8,10 @@ from oracle import gn as ogn
 from oracle import refload
 from oracle import tsdf as ot
 
-pytestmark = [pytest.mark.reference, pytest.mark.skipif(not refload.available(), reason="reference checkout not present")]
+
+def live(test):
+    """the test executes the reference: skipped where no checkout is present"""
+    return pytest.mark.reference(pytest.mark.skipif(not refload.available(), reason="reference checkout not present")(test))
 
 
 def _dq(rng, n, dtype):
@@ -26,6 +29,7 @@ def test_norm3_float32_semantics():
     assert np.array_equal(ref, odq.norm3_like_la(x))
 
 
+@live
 @pytest.mark.parametrize("seed", [0, 1])
 @pytest.mark.parametrize("lw_dtype", [np.float32, np.float64])
 def test_updateTSDF_live(seed, lw_dtype):
@@ -48,6 +52,7 @@ def test_updateTSDF_live(seed, lw_dtype):
     assert np.array_equal(idx[~tie], kd[~tie])
 
 
+@live
 def test_updateTSDF_errors_like_reference():
     f = refload.make_fusion([(0, np.zeros(3, np.float32), np.array([1, 0, 0, 0, 0, 0, 0, 0], np.float32), 1.0)] * 5,
                             np.zeros((2, 2, 2)), np.zeros((2, 2, 2)), 1.0, 4, np.array([1, 0, 0, 0, 0, 0, 0, 0], np.float32))
@@ -57,6 +62,7 @@ def test_updateTSDF_errors_like_reference():
         f.updateTSDF(np.zeros((3, 3)))
 
 
+@live
 def test_fuseDepths_live():
     util, Fusion, FusionDM = refload.load()
     rng = np.random.default_rng(3)
@@ -73,6 +79,7 @@ def test_fuseDepths_live():
     assert np.array_equal(v, rt.ravel()) and np.array_equal(w, rw.ravel()) and m.sum() > 10
 
 
+@live
 def test_computef_live():
     rng = np.random.default_rng(5)
     N, V, k = 20, 50, 4
@@ -109,6 +116,7 @@ def _corr_scene(rng, V=60, L=300, N=20, k=4):
     return node_pos, node_dq, verts, norms, lverts
 
 
+@live
 def test_setupCorrespondences_live():
     """Fusion.setupCorrespondences (clpts branch, core/fusion.py:258-276) with marching cubes replaced by the live vertices."""
     from oracle import graph as og
@@ -132,6 +140,7 @@ def test_setupCorrespondences_live():
     assert (cost < 1).any() and (cost == 1).any()
 
 
+@live
 def test_fusiondm_setupCorrespondences_live():
     """FusionDM.setupCorrespondences (core/fusion_dm.py:219-244): rigid warp by _lw, keeps best_cost <= tolerance."""
     from oracle import graph as og
@@ -154,6 +163,7 @@ def test_fusiondm_setupCorrespondences_live():
     assert np.array_equal(np.array(fdm._correspondences), lverts[best[keep]])
 
 
+@live
 def test_uniform_sample_live():
     from oracle import graph as og
     util, _, _ = refload.load()
@@ -165,6 +175,7 @@ def test_uniform_sample_live():
         assert np.array_equal(ri, oi) and np.array_equal(rv, ov)
 
 
+@live
 def test_update_graph_live():
     """Fusion.update_graph (core/fusion.py:201-239) with marching cubes a no-op: vertex re-linking, unsupported points,
     new nodes initialised by dq_blend, refreshed vertex->node table."""
@@ -199,6 +210,7 @@ def test_update_graph_live():
     assert np.array_equal(np.array(f._neighbor_look_up), look)
 
 
+@live
 def test_fuseDepths_invalid_depth_values_live():
     """NaN, +-inf and positive depth pixels through the unmodified FusionDM.fuseDepths: all skipped (an infinite depth
     becomes NaN in K^-1 * (z*u, z*v, z) for a pinhole K) -- the oracle follows op for op."""
@@ -219,6 +231,7 @@ def test_fuseDepths_invalid_depth_values_live():
     assert 0 < m.sum() < fr.sum() and np.isfinite(rt).all()
 
 
+@live
 def test_fuseDepths_camera_inside_volume_live():
     """Voxels behind the camera (negative projective divisor) and exactly on the camera plane (divisor 0 -> None) through
     the unmodified FusionDM.fuseDepths (core/util.py:312-320 has no sign test)."""
