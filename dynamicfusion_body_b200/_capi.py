@@ -113,6 +113,7 @@ def declare(lib, prefix="dfb_", device=True):
         "point_grid_build": ([C.POINTER(PointGrid), vp, vp, vp, vp], C.c_int),
         "point_grid_knn": ([C.POINTER(PointGrid), vp, C.c_int64, C.c_int, vp, vp, vp], C.c_int),
         "corr_select": ([vp, vp, C.c_int64, vp, vp, C.c_int, vp, vp, vp], C.c_int),
+        "corr_projective": ([vp, vp, C.c_int64, C.POINTER(Views), C.c_double, C.c_double, vp, vp, vp] + ([vp] if device else []), C.c_int),
         "graph_unsupported": ([vp, C.c_int64, vp, C.c_int, vp, vp, vp, vp], C.c_int),
         "graph_sample_rounds": ([C.POINTER(PointGrid), C.c_double, C.c_int, vp, vp, vp], C.c_int),
         "mc_level_scratch_floats": ([], C.c_int64),
@@ -177,7 +178,7 @@ EXPORTS = [
     "dfb_tsdf_update_projective", "dfb_tsdf_update_volume", "dfb_fuse_depth_rigid", "dfb_warp_points", "dfb_dq_blend_points",
     "dfb_gn_residuals", "dfb_gn_residuals_lw", "dfb_gn_pattern_rows", "dfb_gn_pattern_cols", "dfb_gn_normal_eq",
     "dfb_gn_lw_normal_eq", "dfb_gn_solve_workspace_doubles", "dfb_gn_solve",
-    "dfb_point_grid_scratch_ints", "dfb_point_grid_build", "dfb_point_grid_knn", "dfb_corr_select", "dfb_graph_unsupported", "dfb_graph_sample_rounds",
+    "dfb_point_grid_scratch_ints", "dfb_point_grid_build", "dfb_point_grid_knn", "dfb_corr_select", "dfb_corr_projective", "dfb_graph_unsupported", "dfb_graph_sample_rounds",
     "dfb_mc_level_scratch_floats", "dfb_mc_level", "dfb_mc_rows", "dfb_mc_chunks", "dfb_mc_count", "dfb_mc_emit",
     "dfb_knn_brick_count", "dfb_knn_build_volume_radii", "dfb_knn_update_volume", "dfb_brick_nodes_update", "dfb_region_update",
     "dfb_comm_available", "dfb_comm_unique_id", "dfb_comm_init", "dfb_comm_destroy", "dfb_comm_rank", "dfb_comm_world",

@@ -340,6 +340,80 @@ DFB_HDN int project_fuse_ref(const double* lpos, const float* depth, int rows, i
     return 3;
 }
 
+// Projective data association of one warped canonical point w / normal m (float64, from warp_ref) against n_views depth maps
+// (SURVEY 8f rank 1; the contract is oracle/assoc.py).  Per view v, in ascending order: camera frame l = E_v [w,1], ln = R_v m
+// (w, m when E == nullptr); front-facing ln.l < 0; projection as project_fuse_ref plus a one-pixel border ring; the centre depth
+// and its four 4-neighbours valid (> 0) and within max_distance of it; live point c = Kinv [z u, z v, z] at the integer pixel,
+// live normal g = (P(u+1) - P(u-1)) x (P(v+1) - P(v-1)) turned to face the camera; gates |l - c|^2 <= max_distance^2 and
+// ln.g >= min_normal_dot |ln| |g|; cost |ln.(l - c)|, smallest cost wins (strict <: ties keep the lower view).
+// Returns the view (-1: none); cost_out = cost (+inf: none), corr_out = R_v^T (c - t_v) (0: none).
+// depth[v]: [rows][cols] float32, negative depth, 0 = no data.  E: [n_views][12] row-major 3x4 or nullptr.
+DFB_HDN int assoc_projective_ref(const double* w, const double* m, const float* const* depth, int n_views, int rows, int cols,
+                                 const double* K, const double* Kinv, const double* E, double max_distance, double min_normal_dot,
+                                 double* cost_out, double* corr_out) {
+    int best = -1;
+    double best_cost = INFINITY, bc[3] = {0.0, 0.0, 0.0};
+    const double md2 = dmul(max_distance, max_distance);
+    for (int v = 0; v < n_views; ++v) {
+        const double* Ev = E ? E + 12 * v : nullptr;
+        double l[3], ln[3];
+        for (int r = 0; r < 3; ++r) {
+            l[r] = Ev ? dot4_ref(Ev + 4 * r, w[0], w[1], w[2], 1.0) : w[r];
+            ln[r] = Ev ? dot3_ref(Ev + 4 * r, m[0], m[1], m[2]) : m[r];
+        }
+        if (!(dot3_ref(ln, l[0], l[1], l[2]) < 0.0)) continue;
+        const double p0 = dot3_ref(K, l[0], l[1], l[2]);
+        const double p1 = dot3_ref(K + 3, l[0], l[1], l[2]);
+        const double p2 = dot3_ref(K + 6, l[0], l[1], l[2]);
+        if (p2 == 0.0) continue;
+        const double u = ddiv(p0, p2), vv = ddiv(p1, p2);
+        if (!(u >= 0.0 && u < (double)(cols - 1) && vv >= 0.0 && vv < (double)(rows - 1))) continue;
+        const long ui = (long)drint(u), vi = (long)drint(vv);
+        if (ui < 1 || ui > cols - 2 || vi < 1 || vi > rows - 2) continue;
+        const float* D = depth[v];
+        // centre, u-1, u+1, v-1, v+1
+        const long pu[5] = {ui, ui - 1, ui + 1, ui, ui};
+        const long pv[5] = {vi, vi, vi, vi - 1, vi + 1};
+        double z[5];
+        bool ok = true;
+        for (int j = 0; j < 5 && ok; ++j) {
+            z[j] = -1.0 * (double)D[(size_t)pv[j] * cols + pu[j]];
+            ok = z[j] > 0.0 && (j == 0 || fabs(dsub(z[j], z[0])) <= max_distance);
+        }
+        if (!ok) continue;
+        double P[5][3];
+        for (int j = 0; j < 5; ++j) {
+            const double a = dmul(z[j], (double)pu[j]), b = dmul(z[j], (double)pv[j]), c2 = dmul(z[j], 1.0);
+            for (int r = 0; r < 3; ++r) P[j][r] = dot3_ref(Kinv + 3 * r, a, b, c2);
+        }
+        const double* c = P[0];
+        const double du[3] = {dsub(P[2][0], P[1][0]), dsub(P[2][1], P[1][1]), dsub(P[2][2], P[1][2])};
+        const double dv[3] = {dsub(P[4][0], P[3][0]), dsub(P[4][1], P[3][1]), dsub(P[4][2], P[3][2])};
+        double g[3] = {dsub(dmul(du[1], dv[2]), dmul(du[2], dv[1])), dsub(dmul(du[2], dv[0]), dmul(du[0], dv[2])),
+                       dsub(dmul(du[0], dv[1]), dmul(du[1], dv[0]))};
+        const double gc = dot3_ref(g, c[0], c[1], c[2]);
+        if (gc == 0.0) continue;
+        if (gc > 0.0) { g[0] = -g[0]; g[1] = -g[1]; g[2] = -g[2]; }
+        const double d[3] = {dsub(l[0], c[0]), dsub(l[1], c[1]), dsub(l[2], c[2])};
+        if (!(dot3_ref(d, d[0], d[1], d[2]) <= md2)) continue;
+        const double nl = dsqrt(dot3_ref(ln, ln[0], ln[1], ln[2])), ng = dsqrt(dot3_ref(g, g[0], g[1], g[2]));
+        if (!(dot3_ref(ln, g[0], g[1], g[2]) >= dmul(dmul(min_normal_dot, nl), ng))) continue;
+        const double cost = fabs(dot3_ref(ln, d[0], d[1], d[2]));
+        if (!(cost < best_cost)) continue;
+        best = v;
+        best_cost = cost;
+        if (Ev) {
+            const double e[3] = {dsub(c[0], Ev[3]), dsub(c[1], Ev[7]), dsub(c[2], Ev[11])};
+            for (int j = 0; j < 3; ++j) bc[j] = dadd(dadd(dmul(Ev[j], e[0]), dmul(Ev[4 + j], e[1])), dmul(Ev[8 + j], e[2]));
+        } else {
+            bc[0] = c[0]; bc[1] = c[1]; bc[2] = c[2];
+        }
+    }
+    *cost_out = best_cost;
+    corr_out[0] = bc[0]; corr_out[1] = bc[1]; corr_out[2] = bc[2];
+    return best;
+}
+
 // core/util.py:102-137 interpolate_tsdf on a float32 live volume; returns false for "None".
 DFB_HDN bool interpolate_tsdf_ref(const double* pos, const float* t, int rx, int ry, int rz, double* out) {
     const double mn = fmin(fmin(pos[0], pos[1]), pos[2]);

@@ -252,6 +252,29 @@ __global__ void corr_select_kernel(const double* wv, const double* wn, int64_t m
     best_cost[t] = bc;
 }
 
+// Projective data association (dfb_math.h assoc_projective_ref): one thread per warped canonical point, grid-stride.
+__global__ void __launch_bounds__(128) corr_projective_kernel(const double* wv, const double* wn, int64_t m, const dfb_views views,
+                                                              double max_distance, double min_normal_dot, int32_t* view, double* cost,
+                                                              double* corr) {
+    // the camera block is read through pointers by the per-point function: staged in shared memory (indexing the kernel
+    // parameter through a pointer would make every thread copy the whole struct to its local stack)
+    __shared__ double sK[9], sKinv[9], sE[DFB_MAX_VIEWS * 12];
+    __shared__ const float* sD[DFB_MAX_VIEWS];
+    for (int i = threadIdx.x; i < 9; i += blockDim.x) { sK[i] = views.K[i]; sKinv[i] = views.Kinv[i]; }
+    for (int i = threadIdx.x; i < 12 * views.n_views; i += blockDim.x) sE[i] = views.E[i / 12][i % 12];
+    for (int i = threadIdx.x; i < views.n_views; i += blockDim.x) sD[i] = views.depth[i];
+    __syncthreads();
+    for (int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; t < m; t += (int64_t)gridDim.x * blockDim.x) {
+        const double w[3] = {wv[3 * t], wv[3 * t + 1], wv[3 * t + 2]};
+        const double n[3] = {wn[3 * t], wn[3 * t + 1], wn[3 * t + 2]};
+        double c, p[3];
+        view[t] = assoc_projective_ref(w, n, sD, views.n_views, views.rows, views.cols, sK, sKinv, views.has_extrinsics ? sE : nullptr,
+                                       max_distance, min_normal_dot, &c, p);
+        cost[t] = c;
+        corr[3 * t] = p[0]; corr[3 * t + 1] = p[1]; corr[3 * t + 2] = p[2];
+    }
+}
+
 // ---- graph maintenance ----------------------------------------------------------------------------------
 // core/fusion.py:212-215: a surface point is unsupported when min_i |node_i - vert| / dg_w_i >= 1 over its k nearest nodes
 // (float32 difference and norm, then the quotient in float64).
@@ -363,6 +386,24 @@ extern "C" int dfb_corr_select(const double* warped_pts, const double* warped_no
     corr_select_kernel<<<(unsigned)((m + 127) / 128), 128, 0, (cudaStream_t)stream>>>(warped_pts, warped_normals, m, live_verts, nn, k,
                                                                                       best, best_cost);
     DFB_LAUNCH_CHECK("corr_select_kernel");
+    return DFB_OK;
+}
+
+extern "C" int dfb_corr_projective(const double* warped_pts, const double* warped_normals, int64_t m, const dfb_views* views,
+                                   double max_distance, double min_normal_dot, int32_t* view, double* cost, double* corr,
+                                   dfb_stream_t stream) {
+    DFB_REQUIRE(warped_pts && warped_normals && views && view && cost && corr && m >= 0, "null pointer / negative count");
+    DFB_REQUIRE(views->n_views >= 1 && views->n_views <= DFB_MAX_VIEWS, "n_views=%d out of range [1,%d]", views->n_views, DFB_MAX_VIEWS);
+    DFB_REQUIRE(views->rows >= 3 && views->cols >= 3, "depth map %dx%d smaller than 3x3", views->rows, views->cols);
+    for (int v = 0; v < views->n_views; ++v) DFB_REQUIRE(views->depth[v], "depth[%d] is null", v);
+    DFB_REQUIRE(max_distance > 0, "max_distance must be positive");
+    DFB_REQUIRE(min_normal_dot >= -1.0 && min_normal_dot <= 1.0, "min_normal_dot must be in [-1,1]");
+    if (m == 0) return DFB_OK;
+    const int64_t need = (m + 127) / 128;
+    const unsigned blocks = (unsigned)(need < 148 * 16 ? need : 148 * 16);   // 16 blocks per SM, grid-stride beyond
+    corr_projective_kernel<<<blocks, 128, 0, (cudaStream_t)stream>>>(warped_pts, warped_normals, m, *views, max_distance, min_normal_dot,
+                                                                       view, cost, corr);
+    DFB_LAUNCH_CHECK("corr_projective_kernel");
     return DFB_OK;
 }
 

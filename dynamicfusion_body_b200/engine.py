@@ -470,6 +470,22 @@ def corr_select(warped_pts, warped_normals, live_verts, nn):
     return best, cost
 
 
+def corr_projective(warped_pts, warped_normals, views, max_distance, min_normal_dot):
+    """Projective data association of warped canonical points / normals (float64, as `warp_points` returns them) against the
+    depth views of `make_views`: returns (view (m,) int32, -1 = none; cost (m,) float64, +inf = none; corr (m,3) float64, the
+    live point in the frame of the warped points, 0 = none) as CUDA tensors."""
+    dev = warped_pts.device if isinstance(warped_pts, torch.Tensor) and warped_pts.is_cuda else _require_cuda(None)
+    wv = _to_dev(warped_pts, torch.float64, dev).reshape(-1, 3)
+    wn = _to_dev(warped_normals, torch.float64, dev).reshape(-1, 3)
+    m = wv.shape[0]
+    view = torch.empty(m, dtype=torch.int32, device=dev)
+    cost = torch.empty(m, dtype=torch.float64, device=dev)
+    corr = torch.empty((m, 3), dtype=torch.float64, device=dev)
+    _capi.check(_capi.lib().dfb_corr_projective(_ptr(wv), _ptr(wn), m, C.byref(views), float(max_distance), float(min_normal_dot),
+                                                _ptr(view), _ptr(cost), _ptr(corr), _stream()))
+    return view, cost, corr
+
+
 def graph_unsupported(wf, verts, vert_knn):
     """core/fusion.py:211-215: bool (m,) -- surface points no node of `wf` supports."""
     dev = wf.device

@@ -360,6 +360,8 @@ class Fusion(_FusionBase):
         self._subsample_rate = subsample_rate
         self._K = None
         self._Kinv = None
+        self._curr_depths = None        # depth frame of the last projective association (re-associated by solve)
+        self._corridx = None            # vertices the data term covers (None = all of them)
 
     def InitializeCanonicalSpace(self, tsdf=None, depths=None, lws=None, K=None, tsdf_size=256, *, tsdf_shape=None,
                                  slab=None, vertices=None, normals=None, faces=None, nodes=None, radius=None):
@@ -440,12 +442,29 @@ class Fusion(_FusionBase):
             print("Inserted %d new deformation nodes. Current number of deformation nodes: %d" % (len(new_v), self._wf.n_nodes))
         self._set_lookup(self._wf.knn_points(vd, self._knn) if len(new_v) else vknn)
         self._curr_tsdf = None
+        self._curr_depths = None
+        self._corridx = None
         self._correspondences = []
         if self._write_warpfield:
             self.write_warp_field(os.environ.get("DFB_DATA_PATH", "."), 'test')
 
-    def setupCorrespondences(self, curr_tsdf, method='cnn', prune_result=True, tolerance=0.2, *, live_vertices=None):
-        """core/fusion.py:243-313, closest-points branch (the CNN branch is out of scope, so `method` only keeps the
+    def setupCorrespondences(self, curr_tsdf, method='cnn', prune_result=True, tolerance=0.2, *, live_vertices=None, depths=None,
+                             extrinsics=None, max_distance=None, min_normal_dot=0.5):
+        """method='projective': projective data association against depth frames, DynamicFusion's own correspondence step,
+        on the device (include/dfb.h dfb_corr_projective).  Every canonical vertex is warped to the live frame (`_lw` included,
+        with its `_neighbor_look_up` nodes), projected into the views of `depths` ((rows,cols) or (V,rows,cols), host or CUDA,
+        negative depth, 0 = no data, `extrinsics` and the object's K as in `fuseFrame`) and paired with the back-projected pixel
+        it lands on, when that pixel and its four neighbours hold depths within `max_distance` of each other, the pair is closer
+        than `max_distance` and the normals agree (cos >= `min_normal_dot`); the view with the smallest point-to-plane cost wins.
+        `max_distance=None` is the truncation distance, the band in which fuseFrame trusts a measurement.  The canonical normals
+        must point out of the surface, as marching cubes of the TSDF gives them: a vertex counts as visible when its warped
+        normal faces the camera.  `curr_tsdf` and `tolerance` (the closest-point branch's cost bound) are not used.  Vertices
+        without a correspondence are removed with `prune_result=True` (nodes re-linked, as below); with `prune_result=False`
+        every vertex is kept, `_corridx` lists the associated ones and `_correspondences` holds their live points, and the data
+        term of `solve` / `computef` covers those vertices only.  The frame is kept until `update_graph`, so that
+        `solve(method='projective')` can re-associate.
+
+        Any other method: core/fusion.py:243-313, closest-points branch (the CNN branch is out of scope, so `method` only keeps the
         signature; the reference itself takes this branch whenever no TF session exists, :252).  Every canonical vertex
         is warped to the live frame, its k nearest live vertices are searched, and the one with the smallest
         point-to-plane cost |n'.(v' - p)| (< 1, else the nearest) becomes its correspondence.  `live_vertices`
@@ -454,6 +473,13 @@ class Fusion(_FusionBase):
         _neighbor_look_up` and the nodes re-linked (:294-313).  The reference's clpts loop records the wrong index here
         (its inner `for idx in iidx` shadows the vertex index, :269-276, so it deletes the vertex whose number is the
         k-th nearest LIVE vertex's); the intended vertex is pruned instead (stated deviation, like SURVEY Q7)."""
+        if method == 'projective' or depths is not None:
+            if method != 'projective':
+                raise ValueError("depths= is the input of method='projective'")
+            if depths is None:
+                raise ValueError("method='projective' needs depths=")
+            return self._associate_projective(depths, extrinsics, max_distance, min_normal_dot, prune_result)
+        self._corridx = None
         self._curr_tsdf = curr_tsdf
         if self._vertices is None or self._normals is None:
             raise ValueError('canonical vertices/normals have not been set')
@@ -473,6 +499,51 @@ class Fusion(_FusionBase):
             self._normals = np.delete(self._normals, pruned, axis=0)
             self._faces = None
             self._relink_nodes()
+
+    def _associate_projective(self, depths, extrinsics, max_distance, min_normal_dot, prune_result):
+        if self._vertices is None or self._normals is None:
+            raise ValueError('canonical vertices/normals have not been set')
+        if self._K is None:
+            raise ValueError('camera intrinsics K have not been set')
+        d = engine._to_dev(depths, torch.float32, self._device)
+        if d.dim() == 2:
+            d = d[None]
+        if d.dim() != 3:
+            raise ValueError('depth maps must be (rows, cols) or (views, rows, cols)')
+        if extrinsics is not None and len(extrinsics) != d.shape[0]:
+            raise ValueError('length of camera matrix array must equal that of depth maps')
+        md = self._tdist if max_distance is None else float(max_distance)
+        views = engine.make_views(d, self._K, self._Kinv, extrinsics)
+        loc = self._dev(self._neighbor_look_up, torch.int32).reshape(len(self._vertices), -1)
+        wv, wn = engine.warp_points(self._wf, self._lw, self._dev(self._vertices), self._dev(self._normals), idx=loc, k=loc.shape[1])
+        view, cost, corr = engine.corr_projective(wv, wn, views, md, min_normal_dot)
+        hit = (view >= 0).cpu().numpy()
+        if not hit.any():
+            raise ValueError('no canonical vertex is associated with the depth frame')
+        self._curr_depths, self._curr_extrinsics = d, extrinsics
+        self._assoc_args = dict(max_distance=md, min_normal_dot=min_normal_dot, prune_result=prune_result)
+        self._corr_view = view.cpu().numpy()
+        self._corr_cost = cost.cpu().numpy()
+        self._correspondences = corr[torch.from_numpy(hit).to(self._device)].cpu().numpy()
+        if not prune_result:
+            self._corridx = np.nonzero(hit)[0]
+            return
+        self._corridx = None
+        pruned = np.nonzero(~hit)[0]
+        if self._verbose:
+            print('ratio of vertices without a projective correspondence', float(len(pruned)) / float(len(self._vertices)))
+        if len(pruned):
+            self._vertices = np.delete(self._vertices, pruned, axis=0)
+            self._neighbor_look_up = np.delete(np.asarray(self._neighbor_look_up), pruned, axis=0)
+            self._normals = np.delete(self._normals, pruned, axis=0)
+            self._faces = None
+            self._relink_nodes()
+
+    def _reassociate(self):
+        """setupCorrespondences(method='projective') again, against the frame and gates of the last call."""
+        if self._curr_depths is None:
+            raise ValueError("no depth frame on record: call setupCorrespondences(method='projective', depths=...) first")
+        self.setupCorrespondences(None, method='projective', depths=self._curr_depths, extrinsics=self._curr_extrinsics, **self._assoc_args)
 
     # ---- a1 ---------------------------------------------------------------------------------------
     def updateTSDF(self, curr_tsdf=None, wmax=100.0):
@@ -513,6 +584,15 @@ class Fusion(_FusionBase):
         if self._vertices is None or self._normals is None:
             raise ValueError('canonical vertices/normals have not been set')
         corr = np.asarray(self._correspondences, dtype=np.float64)
+        if self._corridx is not None:
+            # data term over the associated vertices only; the regularisation term keeps its neighbours from the full table
+            if len(corr) != len(self._corridx):
+                raise ValueError("Please first call setupCorrespondences to compute point to point correspondences between canonical and live frame vertices!")
+            nlu = self._dev(np.asarray(self._neighbor_look_up), torch.int32).reshape(len(self._vertices), -1)
+            sub = torch.from_numpy(np.asarray(self._corridx, dtype=np.int64)).to(self._device)
+            nvi = torch.from_numpy(np.asarray(self._node_vertex_idx, dtype=np.int64)).to(self._device)
+            return _gn.Problem(self._wf, self._dev(self._vertices)[sub], self._dev(self._normals)[sub], corr, nlu[sub].contiguous(),
+                               self._node_vertex_idx, node_nbr=nlu[nvi].contiguous())
         if len(corr) != len(self._vertices):
             raise ValueError("Please first call setupCorrespondences to compute point to point correspondences between canonical and live frame vertices!")
         nlu = self._neighbor_look_up
@@ -540,9 +620,10 @@ class Fusion(_FusionBase):
         assembled normal equations instead of scipy's finite-difference TRF/LSMR (SURVEY 8a row a12)."""
         if correspondences is not None:
             self._correspondences = correspondences
+            self._corridx = None
             if len(self._correspondences) != len(self._vertices):
                 raise ValueError("Please first call setupCorrespondences to compute point to point correspondences between canonical and live frame vertices!")
-        iteration = 3 if method == 'clpts' else 1
+        iteration = 3 if method in ('clpts', 'projective') else 1
         self._itercounter += 1
         opts = dict(gn_options or {})
         prob = self._problem()
@@ -554,10 +635,16 @@ class Fusion(_FusionBase):
             if method == 'clpts' and (correspondences is None or self._curr_tsdf is not None):
                 self.setupCorrespondences(self._curr_tsdf, method='clpts')
                 prob = self._problem()
+            elif method == 'projective' and (correspondences is None or self._curr_depths is not None):
+                self._reassociate()                                       # same rule against the depth frame on record
+                prob = self._problem()
         rw = regularization_weight
         for it in range(iteration):
             if it > 0 and correspondences is None:
-                self.setupCorrespondences(self._curr_tsdf, method='clpts')
+                if method == 'projective':
+                    self._reassociate()
+                else:
+                    self.setupCorrespondences(self._curr_tsdf, method='clpts')
                 prob = self._problem()
             x0 = self._wf.node_dq.double().reshape(-1)
             res = prob.gauss_newton(x0, self._lw, rw, max_iter=gn_iterations, huber=opts.get("huber", True),

@@ -58,7 +58,10 @@ class GNResult:
 class Problem:
     """Device-resident least-squares problem: vertices, normals, correspondences, vertex->node kNN, nodes."""
 
-    def __init__(self, wf, vertices, normals, corr, vert_knn, node_vertex_idx, shard=None, reg_owner=True):
+    def __init__(self, wf, vertices, normals, corr, vert_knn, node_vertex_idx, shard=None, reg_owner=True, *, node_nbr=None):
+        """node_nbr (optional, (N,k)): the regularisation neighbours of every node.  Default: vert_knn[node_vertex_idx]
+        (core/fusion.py:477), which needs vert_knn to cover every vertex; a problem over a subset of the vertices (the data term
+        of the associated ones only) passes the rows of the full vertex->node table here."""
         dev = wf.device
         self.wf = wf
         self.device = dev
@@ -70,7 +73,9 @@ class Problem:
         self.n_vert = int(self.vertices.shape[0])
         self.n_nodes = wf.n_nodes
         nvi = np.asarray(node_vertex_idx, dtype=np.int64)
-        if isinstance(vert_knn, torch.Tensor):
+        if node_nbr is not None:
+            self.node_nbr = _to_dev(node_nbr, torch.int32, dev).reshape(self.n_nodes, self.k)
+        elif isinstance(vert_knn, torch.Tensor):
             self.node_nbr = self.vert_knn[torch.from_numpy(nvi).to(dev)].contiguous()
         else:
             self.node_nbr = _to_dev(np.asarray(vert_knn)[nvi], torch.int32, dev).reshape(self.n_nodes, self.k)

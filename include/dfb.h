@@ -239,6 +239,15 @@ int dfb_point_grid_knn(const dfb_point_grid* g, const double* queries, int64_t m
  * live_verts, best_cost [m] = min(1, min_j |n . (v - p_j)|) with the reference's first-neighbour default. */
 int dfb_corr_select(const double* warped_pts, const double* warped_normals, int64_t m, const float* live_verts,
                     const int32_t* nn, int k, int32_t* best, double* best_cost, dfb_stream_t stream);
+/* Projective data association (SURVEY 8f rank 1, DynamicFusion's correspondence step) of warped canonical points /
+ * normals [m][3] (from dfb_warp_points) against the depth views: view [m] (-1 = none), cost [m], corr [m][3].
+ * Per view: camera frame through E_v, front-facing test, projection and rounding as dfb_tsdf_update_projective, a one-pixel
+ * border ring excluded, centre and 4-neighbour depths valid and within max_distance of each other, live point and normal
+ * from the back-projected pixels, gates |l - c| <= max_distance and ln.g >= min_normal_dot |ln| |g|, cost |ln.(l - c)|
+ * (smallest wins, ties to the lower view); corr = R_v^T (c - t_v) in the frame of the warped points (oracle/assoc.py). */
+int dfb_corr_projective(const double* warped_pts, const double* warped_normals, int64_t m, const dfb_views* views,
+                        double max_distance, double min_normal_dot, int32_t* view, double* cost, double* corr,
+                        dfb_stream_t stream);
 /* core/fusion.py:211-215: unsupported [m] = 1 where min over the k nearest nodes of |node - vert| / dg_w >= 1. */
 int dfb_graph_unsupported(const float* verts, int64_t m, const int32_t* vert_knn, int k, const float* node_pos,
                           const float* node_w, uint8_t* unsupported, dfb_stream_t stream);
