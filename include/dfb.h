@@ -201,14 +201,19 @@ int dfb_gn_residuals_lw(const dfb_gn_problem* prob, const double* node_dq, int d
 int dfb_gn_pattern_rows(const dfb_gn_problem* prob, uint32_t* bitmap, int32_t* row_ptr, dfb_stream_t stream);
 int dfb_gn_pattern_cols(int n_nodes, const uint32_t* bitmap, const int32_t* row_ptr, int32_t* col_idx, dfb_stream_t stream);
 /* Analytic Jacobian -> BSR normal equations H = J^T W J [nnzb][8][8], g = J^T W f [N][8], cost[0] = robust cost,
- * cost[1] = 0.5 |f|^2 (all zeroed first).  Replaces scipy's finite-difference Jacobian (core/fusion.py:382-392). */
+ * cost[1] = 0.5 |f|^2 (all zeroed first).  Replaces scipy's finite-difference Jacobian (core/fusion.py:382-392).
+ * BSR contract (here and in dfb_gn_solve): the columns of every row ascend, every diagonal block (i, i) is present, and the
+ * pattern is symmetric and holds every node pair of the problem -- dfb_gn_pattern_* produce exactly that.  Blocks are looked up
+ * by binary search; a missing block is NOT detected: its contribution lands in a wrong slot. */
 int dfb_gn_normal_eq(const dfb_gn_problem* prob, const double* x, const int32_t* row_ptr, const int32_t* col_idx, int64_t nnzb,
                      double* H, double* g, double* cost, dfb_stream_t stream);
 /* 8x8 normal equations of the rigid fit (core/fusion.py:356-360): H8 [64], g8 [8], cost [2] on the device. */
 int dfb_gn_lw_normal_eq(const dfb_gn_problem* prob, const double* node_dq, const double* lw, double* H8, double* g8, double* cost,
                         dfb_stream_t stream);
 /* Damped node-space solve (H + lambda*mean(diag H)*I) delta = -g by block-Jacobi PCG, then x_new = x + delta.
- * workspace: dfb_gn_solve_workspace_doubles(N) doubles; workspace[0..7] = {mu, final (r,z), -, -, initial (r,z), -, iterations, trace}. */
+ * H: BSR as for dfb_gn_normal_eq, and symmetric (CG).  The solve stops once (r,z) <= tol^2 (r0,z0) or after max_iter updates.
+ * workspace: dfb_gn_solve_workspace_doubles(N) doubles; workspace[0..7] = {mu, final (r,z), -, -, initial (r,z), -, iterations, trace},
+ * where iterations = the number of updates of delta applied (every kernel variant counts the same way). */
 int64_t dfb_gn_solve_workspace_doubles(int n_nodes);
 int dfb_gn_solve(int n_nodes, const int32_t* row_ptr, const int32_t* col_idx, const double* H, const double* g, double lambda,
                  int max_iter, double tol, const double* x, double* x_new, double* delta, double* workspace, dfb_stream_t stream);

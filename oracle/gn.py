@@ -22,15 +22,17 @@ def reg_neighbours(vert_knn, node_vertex_idx):
     return np.asarray(vert_knn)[np.asarray(node_vertex_idx)]
 
 
-def computef(x, vertices, normals, corr, vert_knn, node_pos, node_w, node_vertex_idx, lw, rw):
-    """core/fusion.py:459-491.  x (8N,) (its dtype matters exactly like in the reference: `dqs = np.split(x, ...)`)."""
+def computef(x, vertices, normals, corr, vert_knn, node_pos, node_w, node_vertex_idx, lw, rw, node_nbr=None):
+    """core/fusion.py:459-491.  x (8N,) (its dtype matters exactly like in the reference: `dqs = np.split(x, ...)`).
+    node_nbr (N,k): regularisation neighbours of every node (default reg_neighbours(vert_knn, node_vertex_idx)); a problem over a
+    subset of the vertices passes the rows of the full vertex->node table, like gn.Problem(node_nbr=)."""
     x = np.asarray(x)
     dqs = x.reshape(-1, 8)
     n_nodes = len(dqs)
     node_w = np.broadcast_to(np.asarray(node_w, dtype=np.float64), (n_nodes,))
     vw, nw = _dq.warp(vertices, node_pos[vert_knn], dqs[vert_knn], node_w[vert_knn], lw=lw, normal=normals)
     f_data = np.einsum('ij,ij->i', nw, vw - corr)
-    nbr = reg_neighbours(vert_knn, node_vertex_idx)              # (N,k)
+    nbr = reg_neighbours(vert_knn, node_vertex_idx) if node_nbr is None else np.asarray(node_nbr)   # (N,k)
     k = nbr.shape[1]
     pj = node_pos[nbr]                                           # (N,k,3) dgj_v
     di = _dq.dqb_warp(dqs[:, None, :], pj)                       # dqb_warp(dgi_se3, dgj_v)
@@ -148,8 +150,8 @@ def data_jacobian_parts(x, vertices, normals, corr, vert_knn, node_pos, node_w, 
     return r, g, wts
 
 
-def jacobian(x, vertices, normals, corr, vert_knn, node_pos, node_w, node_vertex_idx, lw, rw):
-    """Sparse analytic Jacobian (CSR, rows V + 3kN, cols 8N) of computef and its residual vector."""
+def jacobian(x, vertices, normals, corr, vert_knn, node_pos, node_w, node_vertex_idx, lw, rw, node_nbr=None):
+    """Sparse analytic Jacobian (CSR, rows V + 3kN, cols 8N) of computef and its residual vector.  node_nbr: as in computef."""
     from scipy.sparse import csr_matrix
     dqs = np.asarray(x, dtype=np.float64).reshape(-1, 8)
     n_nodes = len(dqs)
@@ -160,7 +162,7 @@ def jacobian(x, vertices, normals, corr, vert_knn, node_pos, node_w, node_vertex
     rows = np.repeat(np.arange(V), k * 8)
     cols = (vert_knn[:, :, None] * 8 + np.arange(8)[None, None, :]).reshape(-1)
     vals = (wts[:, :, None] * g[:, None, :]).reshape(-1)
-    nbr = reg_neighbours(vert_knn, node_vertex_idx)
+    nbr = reg_neighbours(vert_knn, node_vertex_idx) if node_nbr is None else np.asarray(node_nbr)
     pj = node_pos.astype(np.float64)[nbr]                        # (N,k,3)
     c = rw * np.maximum(node_wa[:, None], node_wa[nbr])          # (N,k)
     Ji = c[..., None, None] * dW_dq(dqs[:, None, :], pj)         # (N,k,3,8)
@@ -218,12 +220,16 @@ def robust_cost(f, f_scale=1.0, huber=True):
     return 0.5 * f_scale ** 2 * float(np.where(z <= 1, z, 2 * np.sqrt(z) - 1).sum())
 
 
-def normal_equations(J, f, f_scale=1.0, huber=True):
+def normal_equations(J, f, f_scale=1.0, huber=True, dense=True):
+    """H = J^T W J, g = J^T W f.  dense=False returns H as a scipy CSR (sorted indices, duplicates summed): at 5 k nodes the
+    dense matrix is 40 k^2 doubles."""
     w = huber_weights(f, f_scale, huber)
     JW = J.multiply(w[:, None]).tocsr()
-    H = (J.T @ JW).toarray()
+    H = (J.T.tocsr() @ JW).tocsr()
+    H.sum_duplicates()
+    H.sort_indices()
     g = np.asarray(J.T @ (w * f)).ravel()
-    return H, g
+    return (H.toarray() if dense else H), g
 
 
 def gn_step(H, g, lam):
@@ -233,22 +239,74 @@ def gn_step(H, g, lam):
     return np.linalg.solve(H + mu * np.eye(n), -g)
 
 
+def _damping(H, lam):
+    return lam * H.diagonal().sum() / H.shape[0]
+
+
+def sparse_gn_step(H, g, lam):
+    """gn_step for a scipy sparse H, by a sparse LU of H + mu I."""
+    from scipy.sparse import identity
+    from scipy.sparse.linalg import splu
+    n = H.shape[0]
+    A = (H + _damping(H, lam) * identity(n, format="csr")).tocsc()
+    return splu(A).solve(-np.asarray(g, dtype=np.float64))
+
+
+def pcg_block_jacobi(H, g, lam, tol, max_iter):
+    """float64 restatement of the device solve dfb_gn_solve: (H + mu I) delta = -g with mu = lam * trace(H) / (8N), conjugate
+    gradients preconditioned by the inverses of the damped 8x8 diagonal blocks, starting at delta = 0, stopping once
+    (r, z) <= tol^2 (r0, z0) or after max_iter updates.  Returns (delta, number of updates applied) -- the count the device
+    reports in workspace[6].  H: scipy sparse (8N, 8N) or dense."""
+    from scipy.sparse import csr_matrix
+    H = csr_matrix(H)
+    n8 = H.shape[0]
+    n = n8 // 8
+    mu = _damping(H, lam)
+    C = H.tocoo()
+    on = (C.row // 8) == (C.col // 8)
+    D = np.zeros((n, 8, 8))
+    np.add.at(D, (C.row[on] // 8, C.row[on] % 8, C.col[on] % 8), C.data[on])
+    Minv = np.linalg.inv(D + mu * np.eye(8))
+
+    def prec(v):
+        return np.einsum("iab,ib->ia", Minv, v.reshape(n, 8)).reshape(-1)
+
+    delta = np.zeros(n8)
+    r = -np.asarray(g, dtype=np.float64)
+    z = prec(r)
+    p = z.copy()
+    rz = rz0 = float(r @ z)
+    it = 0
+    while it < max_iter and rz > tol * tol * rz0:
+        q = H @ p + mu * p
+        alpha = rz / float(p @ q)
+        delta += alpha * p
+        r -= alpha * q
+        z = prec(r)
+        rz_new = float(r @ z)
+        p = z + (rz_new / rz) * p
+        rz = rz_new
+        it += 1
+    return delta, it
+
+
 def gauss_newton_loop(x0, vertices, normals, corr, vert_knn, node_pos, node_w, node_vertex_idx, lw, rw, max_iter=15, huber=True, f_scale=1.0,
-                      lam0=1e-3, lam_min=1e-5):
+                      lam0=1e-3, lam_min=1e-5, sparse=False):
     """The damped Gauss-Newton (Levenberg-Marquardt accept / reject) iteration of dynamicfusion_body_b200.gn.Problem.gauss_newton with
     every linear system solved densely in float64 -- the oracle of the PRODUCT's optimiser loop (the reference hands `computef` to
-    scipy's TRF, whose trajectory is not a parity target: SURVEY 8a row a12).  Returns (x, cost0, cost, accepted)."""
+    scipy's TRF, whose trajectory is not a parity target: SURVEY 8a row a12).  Returns (x, cost0, cost, accepted).
+    sparse=True: the same systems through scipy sparse matrices and a sparse LU (sparse_gn_step), for graphs of thousands of nodes."""
     x = np.asarray(x0, dtype=np.float64).copy()
 
     def assemble(xx):
         J, f = jacobian(xx, vertices, normals, corr, vert_knn, node_pos, node_w, node_vertex_idx, lw, rw)
-        H, g = normal_equations(J, f, f_scale, huber)
+        H, g = normal_equations(J, f, f_scale, huber, dense=not sparse)
         return H, g, robust_cost(f, f_scale, huber)
 
     H, g, cost = assemble(x)
     cost0, lam, accepted = cost, lam0, 0
     for _ in range(max_iter):
-        x_new = x + gn_step(H, g, lam)
+        x_new = x + (sparse_gn_step(H, g, lam) if sparse else gn_step(H, g, lam))
         H2, g2, cost_new = assemble(x_new)
         if np.isfinite(cost_new) and cost_new < cost:
             x, H, g, cost = x_new, H2, g2, cost_new
