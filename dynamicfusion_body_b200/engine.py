@@ -486,6 +486,55 @@ def corr_projective(warped_pts, warped_normals, views, max_distance, min_normal_
     return view, cost, corr
 
 
+def camera_views(K, rows, cols, extrinsics=None, n_views=None):
+    """dfb_views of cameras without depth maps (the input of `render`): intrinsics K, image size, and either `n_views` copies of
+    the camera (default 1) or one view per 3x4 extrinsic of `extrinsics` (world -> camera, as in `make_views`)."""
+    K = np.asarray(K, dtype=np.float64)
+    v = _capi.Views()
+    v.n_views = (1 if n_views is None else int(n_views)) if extrinsics is None else len(extrinsics)
+    if not 1 <= v.n_views <= _capi.DFB_MAX_VIEWS:
+        raise ValueError("between 1 and %d views per pass" % _capi.DFB_MAX_VIEWS)
+    v.rows, v.cols = int(rows), int(cols)
+    Kinv = np.linalg.inv(K)
+    for i in range(9):
+        v.K[i] = float(K.ravel()[i])
+        v.Kinv[i] = float(Kinv.ravel()[i])
+    v.has_extrinsics = 0 if extrinsics is None else 1
+    if extrinsics is not None:
+        E = np.asarray(extrinsics, dtype=np.float64).reshape(v.n_views, 12)
+        for j in range(v.n_views):
+            for i in range(12):
+                v.E[j][i] = float(E[j, i])
+    return v
+
+
+def render_workspace(n_faces, views, device=None):
+    """The caller-owned workspace of `render` (dfb_render_workspace_words uint64 words, held as int64); after a call, element 0
+    counts the (face, view) pairs that went through the large-face kernel."""
+    words = _capi.lib().dfb_render_workspace_words(int(n_faces), views.n_views, views.rows, views.cols)
+    if words < 0:
+        raise ValueError("invalid render geometry: %d faces, %d views of %dx%d" % (n_faces, views.n_views, views.rows, views.cols))
+    return torch.empty(words, dtype=torch.int64, device=_require_cuda(device))
+
+
+def render(pts, faces, views, workspace=None):
+    """Z-buffer rendering of the mesh pts (n,3) (float64, e.g. as `warp_points` returns it) / faces (f,3) int32 into the views of
+    `camera_views` or `make_views` (their depth maps are not read).  Returns CUDA tensors depth (V,rows,cols) float32 (negative
+    depth, 0 = no face: ready for `update_projective` / `corr_projective`), face (V,rows,cols) int32 (-1 = none) and normal
+    (V,rows,cols,3) float32 (the face's unit normal in the frame of pts, 0 = none).  `workspace`: from `render_workspace`."""
+    dev = pts.device if isinstance(pts, torch.Tensor) and pts.is_cuda else _require_cuda(None)
+    p = _to_dev(pts, torch.float64, dev).reshape(-1, 3)
+    f = _to_dev(faces, torch.int32, dev).reshape(-1, 3)
+    V, rows, cols = views.n_views, views.rows, views.cols
+    ws = render_workspace(f.shape[0], views, dev) if workspace is None else workspace
+    depth = torch.empty((V, rows, cols), dtype=torch.float32, device=dev)
+    face = torch.empty((V, rows, cols), dtype=torch.int32, device=dev)
+    normal = torch.empty((V, rows, cols, 3), dtype=torch.float32, device=dev)
+    _capi.check(_capi.lib().dfb_render(_ptr(p), p.shape[0], _ptr(f), f.shape[0], C.byref(views), _ptr(ws), ws.numel(),
+                                       _ptr(depth), _ptr(face), _ptr(normal), _stream()))
+    return depth, face, normal
+
+
 def graph_unsupported(wf, verts, vert_knn):
     """core/fusion.py:211-215: bool (m,) -- surface points no node of `wf` supports."""
     dev = wf.device

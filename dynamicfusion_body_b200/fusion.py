@@ -17,6 +17,7 @@ The callers either side of the hot paths (SURVEY 8f ranks 1-2) run on the device
 (closest-point correspondences), `update_graph` / `construct_graph` (node sampling, unsupported surface points,
 vertex->node tables), and so does surface extraction (8f rank 3, `marching_cubes`; `surface_extractor` swaps it out).
 """
+import collections
 import os
 
 import numpy as np
@@ -26,6 +27,9 @@ from scipy.spatial import KDTree
 from . import _capi, engine
 from . import dist as ddist
 from . import gn as _gn
+
+
+LiveRender = collections.namedtuple("LiveRender", ["depth", "normal", "face", "vertices", "faces"])
 
 
 def _as_np(a):
@@ -578,6 +582,35 @@ class Fusion(_FusionBase):
             raise ValueError('length of camera matrix array must equal that of depth maps')
         return engine.update_projective(self._vol, self._wf, self._lw, d, self._K, self._Kinv, extrinsics, self._tdist, wmax,
                                         mode=self._mode if mode is None else mode, want_masks=want_masks)
+
+    def render_live(self, K=None, extrinsics=None, rows=480, cols=640):
+        """The canonical model warped into the live frame and rendered from the live cameras, on the device (include/dfb.h
+        dfb_render): DynamicFusion's view of what it reconstructed, to compare with the input depth.  The canonical surface is
+        extracted as `write_canonical_mesh` extracts it (step 1, the same level), each vertex is warped by the current field with
+        its k nearest nodes and `_lw`, and the mesh is rasterised into one view per 3x4 extrinsic of `extrinsics` (one view without;
+        K defaults to the object's, as in `fuseFrame`).  Returns LiveRender(depth (V,rows,cols) float32, negative depth, 0 = no
+        surface, the convention `fuseFrame` and `setupCorrespondences(method='projective')` take; normal (V,rows,cols,3) float32,
+        the face normal in the live frame; face (V,rows,cols) int32, -1 = none; vertices (n,3) float32 and faces (f,3) int32, the
+        canonical mesh the face ids index) as CUDA tensors.  An empty volume renders empty maps.  On a volume sharded over the
+        process group every rank receives the whole mesh and renders the whole image (not exercised on more than one GPU)."""
+        K = self._K if K is None else np.asarray(K, dtype=np.float64)
+        if K is None:
+            raise ValueError('camera intrinsics K have not been set')
+        if self._vol is None:
+            raise ValueError('the canonical volume has not been initialised')
+        views = engine.camera_views(K, rows, cols, extrinsics)
+        verts, faces, _, _ = self._device_surface(1, None, keep_on_device=True)
+        verts = engine._to_dev(verts, torch.float32, self._device).reshape(-1, 3)
+        faces = engine._to_dev(faces, torch.int32, self._device).reshape(-1, 3)
+        if len(faces) and self._wf.n_nodes:
+            idx = self._wf.knn_points(verts, self._knn)
+            live = engine.warp_points(self._wf, self._lw, verts, idx=idx, k=self._knn)
+        elif len(faces):
+            raise ValueError('the deformation graph has no nodes to warp the canonical surface with')
+        else:
+            live = torch.zeros((0, 3), dtype=torch.float64, device=self._device)
+        depth, face, normal = engine.render(live, faces, views)
+        return LiveRender(depth, normal, face, verts, faces)
 
     # ---- solve (core/fusion.py:327-491) -------------------------------------------------------------
     def _problem(self):

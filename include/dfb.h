@@ -253,6 +253,18 @@ int dfb_corr_select(const double* warped_pts, const double* warped_normals, int6
 int dfb_corr_projective(const double* warped_pts, const double* warped_normals, int64_t m, const dfb_views* views,
                         double max_distance, double min_normal_dot, int32_t* view, double* cost, double* corr,
                         dfb_stream_t stream);
+/* Z-buffer rasteriser (the reference's GL vertex-id / depth renderer, core/gl/glrender.py, without a GL context): the mesh
+ * pts [n_pts][3] float64 (e.g. warped by dfb_warp_points) / faces [n_faces][3] int32 seen by the cameras of *views (K, E,
+ * rows, cols; its depth[] pointers are ignored).  Per view v, each [rows][cols], pixel (r, c) sampled at x = c, y = r:
+ * depth (negative depth, 0 = no face: the convention of every depth input here), face (id, -1 = none) and normal [..][3]
+ * (the winning face's unit normal (Pb - Pa) x (Pc - Pa) in the frame of pts, float32; 0 = none or degenerate).  Faces with
+ * an index outside [0, n_pts), a vertex at camera depth <= 0 or zero projected area are culled; edges are inclusive, depth
+ * is perspective-correct, the nearest float32 depth wins and ties go to the lower face id (oracle/render.py).
+ * workspace: dfb_render_workspace_words(n_faces, n_views, rows, cols) uint64 words (-1 for invalid arguments); after the
+ * call workspace[0] holds the number of (face, view) pairs that went through the large-face kernel. */
+int64_t dfb_render_workspace_words(int64_t n_faces, int n_views, int rows, int cols);
+int dfb_render(const double* pts, int64_t n_pts, const int32_t* faces, int64_t n_faces, const dfb_views* views,
+               uint64_t* workspace, int64_t workspace_words, float* depth, int32_t* face, float* normal, dfb_stream_t stream);
 /* core/fusion.py:211-215: unsupported [m] = 1 where min over the k nearest nodes of |node - vert| / dg_w >= 1. */
 int dfb_graph_unsupported(const float* verts, int64_t m, const int32_t* vert_knn, int k, const float* node_pos,
                           const float* node_w, uint8_t* unsupported, dfb_stream_t stream);
