@@ -2,8 +2,10 @@
 
 torch is used for what it is good at here -- owning device memory, streams, and (in dist.py)
 torch.distributed -- never for the arithmetic of the hot path.  Every function below ends in a call
-into libdfb_b200.so on the current CUDA stream; there is no eager/torch/CPU fallback.
+into libdfb_b200.so on the current CUDA stream; there is no eager/torch/CPU fallback.  (`track_rigid` and `se3_exp` are the
+host-side Levenberg-Marquardt loop around such calls: a 6x6 solve per iteration.)
 """
+import collections
 import ctypes as C
 import os
 
@@ -533,6 +535,121 @@ def render(pts, faces, views, workspace=None):
     _capi.check(_capi.lib().dfb_render(_ptr(p), p.shape[0], _ptr(f), f.shape[0], C.byref(views), _ptr(ws), ws.numel(),
                                        _ptr(depth), _ptr(face), _ptr(normal), _stream()))
     return depth, face, normal
+
+
+TRACK_SUMS = 29
+TrackResult = collections.namedtuple("TrackResult", ["lw", "cost", "pixels", "iterations", "converged", "residual"], defaults=(None,))
+TrackResult.__doc__ = """Result of `track_rigid`: lw (3,4) float64 world -> camera with an orthonormal rotation; cost, the mean Huber
+cost per contributing pixel at lw on the finest level; pixels, their number; iterations, one count per level; converged, whether
+the finest level ended on a negligible step rather than on its iteration budget; residual, the finest level's residual map when
+it was asked for (`FusionDM.track(want_residual=True)`), else None."""
+
+
+def _volume_struct(vol):
+    """dfb_volume of a DeviceVolume, or of a (tsdf, weight) pair of whole float32 CUDA volumes read in place."""
+    if isinstance(vol, DeviceVolume):
+        return vol.struct()
+    tsdf, weight = vol
+    if not (tsdf.is_cuda and weight.is_cuda and tsdf.dtype == torch.float32 and weight.dtype == torch.float32):
+        raise ValueError("device volumes must be float32 CUDA tensors")
+    if tsdf.dim() != 3 or tuple(tsdf.shape) != tuple(weight.shape) or not (tsdf.is_contiguous() and weight.is_contiguous()):
+        raise ValueError("tsdf and weight must be contiguous 3-D volumes of the same shape")
+    s = _capi.Volume()
+    s.tsdf, s.weight = tsdf.data_ptr(), weight.data_ptr()
+    s.rx, s.ry, s.rz = (int(r) for r in tsdf.shape)
+    s.x0, s.x1 = 0, s.rx
+    return s
+
+
+def track_normal_eq(vol, tsdf_res, depth, lw34, K, Kinv, scale, center, stride, tdist, delta, workspace=None, want_residual=False):
+    """dfb_track_normal_eq: the 29 sums (numpy float64: H upper triangle, g, Huber cost, pixel count) of the depth frame `depth`
+    (CUDA (rows, cols) float32, negative depth) at the pose lw34 (world -> camera) against the whole volume `vol` (a DeviceVolume
+    or a (tsdf, weight) pair of float32 CUDA tensors), and, with want_residual, the residual map (ceil(rows/stride),
+    ceil(cols/stride)) float64 CUDA tensor (NaN where a pixel did not contribute).  `workspace`: a float64 CUDA tensor of at least
+    dfb_track_workspace_doubles elements (allocated when None)."""
+    assert depth.is_cuda and depth.dtype == torch.float32 and depth.is_contiguous() and depth.dim() == 2
+    rows, cols = depth.shape
+    f64 = _capi.c_f64p
+    K = np.ascontiguousarray(K, dtype=np.float64)
+    Kinv = np.ascontiguousarray(np.linalg.inv(K) if Kinv is None else Kinv, dtype=np.float64)
+    lw34 = np.ascontiguousarray(lw34, dtype=np.float64).reshape(12)
+    center = np.ascontiguousarray(np.zeros(3) if center is None else center, dtype=np.float64).reshape(3)
+    if workspace is None:
+        n = int(_capi.lib().dfb_track_workspace_doubles(rows, cols, int(stride)))
+        workspace = torch.empty(max(n, 1), dtype=torch.float64, device=depth.device)
+    out = torch.empty(TRACK_SUMS, dtype=torch.float64, device=depth.device)
+    res = None
+    if want_residual:
+        res = torch.empty(((rows + stride - 1) // stride, (cols + stride - 1) // stride), dtype=torch.float64, device=depth.device)
+    v = _volume_struct(vol)
+    _capi.check(_capi.lib().dfb_track_normal_eq(C.byref(v), int(tsdf_res), float(scale), center.ctypes.data_as(f64), _ptr(depth),
+                                                rows, cols, K.ctypes.data_as(f64), Kinv.ctypes.data_as(f64), lw34.ctypes.data_as(f64),
+                                                int(stride), float(tdist), float(delta), _ptr(workspace), workspace.numel(), _ptr(out),
+                                                _ptr(res), _stream()))
+    sums = out.cpu().numpy()
+    return (sums, res) if want_residual else sums
+
+
+def _unpack_sums(sums):
+    sums = np.asarray(sums, dtype=np.float64)
+    H = np.zeros((6, 6))
+    H[np.triu_indices(6)] = sums[:21]
+    H = H + np.triu(H, 1).T
+    return H, sums[21:27], float(sums[27]), int(round(float(sums[28])))
+
+
+def se3_exp(xi):
+    """Exp of the twist xi = (tau, omega) (Rodrigues): the rotation and translation of x -> R x + t."""
+    xi = np.asarray(xi, dtype=np.float64)
+    tau, om = xi[:3], xi[3:]
+    th = float(np.linalg.norm(om))
+    W = np.array([[0.0, -om[2], om[1]], [om[2], 0.0, -om[0]], [-om[1], om[0], 0.0]])
+    W2 = W @ W
+    if th < 1e-4:
+        A, B, Cc = 1.0 - th * th / 6.0, 0.5 - th * th / 24.0, 1.0 / 6.0 - th * th / 120.0
+    else:
+        A, B, Cc = np.sin(th) / th, (1.0 - np.cos(th)) / th ** 2, (th - np.sin(th)) / th ** 3
+    Rm = np.eye(3) + A * W + B * W2
+    V = np.eye(3) + B * W + Cc * W2
+    return Rm, V @ tau
+
+
+def track_rigid(normal_eq, lw0, strides=(4, 2, 1), iterations=10, lam0=1e-4, min_pixels=100, scale=1.0):
+    """Levenberg-Marquardt on the rigid camera pose, coarse to fine.  `normal_eq(lw, stride)` returns the 29 sums of
+    dfb_track_normal_eq for the 3x4 world -> camera pose lw (the device's `track_normal_eq` or the oracle's `normal_eq`: both
+    backends run this same loop).  Starting from lw0, for each stride in `strides` (a sampling step standing in for an image
+    pyramid), at most `iterations` times: solve (H + lam mean(diag H) I) xi = -g, move the camera-to-world pose P = lw^-1 to
+    Exp(xi) P exactly (`se3_exp`), and accept the step when the mean Huber cost (cost / count) does not rise and at least
+    `min_pixels` pixels still contribute; an accepted step divides lam by 10, a rejected one multiplies it by 10.
+    A level ends on a step with |omega| < 1e-6 and |tau| < 1e-6 scale (scale: the volume's voxel size, world units).  Each level
+    starts from lam0 and raises ValueError when fewer than `min_pixels` pixels contribute at its start.  strides, iterations,
+    lam0 and min_pixels are starting values, not tuned ones.  Returns TrackResult."""
+    lw = np.asarray(lw0, dtype=np.float64).reshape(3, 4).copy()
+    Rc = lw[:, :3].T.copy()
+    Cc = -Rc @ lw[:, 3]
+    iters, converged, cost, n = [], False, 0.0, 0
+    for s in strides:
+        H, g, cost, n = _unpack_sums(normal_eq(lw, s))
+        if n < min_pixels:
+            raise ValueError("only %d pixels of the frame meet the fused surface at stride %d (at least %d needed)" % (n, s, min_pixels))
+        lam, it, converged = lam0, 0, False
+        while it < iterations:
+            it += 1
+            xi = np.linalg.solve(H + lam * np.mean(np.diag(H)) * np.eye(6), -g)
+            dR, dt = se3_exp(xi)
+            Rn, Cn = dR @ Rc, dR @ Cc + dt
+            lwn = np.concatenate([Rn.T, (-Rn.T @ Cn)[:, None]], 1)
+            Hn, gn, costn, nn = _unpack_sums(normal_eq(lwn, s))
+            if nn >= min_pixels and costn / nn <= cost / n:
+                Rc, Cc, lw, H, g, cost, n = Rn, Cn, lwn, Hn, gn, costn, nn
+                lam /= 10.0
+            else:
+                lam *= 10.0
+            if np.linalg.norm(xi[3:]) < 1e-6 and np.linalg.norm(xi[:3]) < 1e-6 * scale:
+                converged = True
+                break
+        iters.append(it)
+    return TrackResult(lw, cost / n, n, tuple(iters), converged)
 
 
 def graph_unsupported(wf, verts, vert_knn):

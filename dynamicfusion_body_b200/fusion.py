@@ -737,6 +737,44 @@ class FusionDM(_FusionBase):
             return (tsdf, tsdf_w)
         return (out_t, out_w)
 
+    def track(self, dm, lw, tsdf=None, tsdf_w=None, scale=1.0, center=np.zeros(3), *, strides=(4, 2, 1), iterations=10, delta=None,
+              min_pixels=100, want_residual=False):
+        """The camera pose of the depth frame `dm` (negative depth, 0 = no data) against the fused volume, from the initial pose
+        `lw` (3x4 world -> camera, the `lw` of fuseDepths; typically the previous frame's): rigid point-to-TSDF alignment on the
+        device (include/dfb.h dfb_track_normal_eq, Levenberg-Marquardt in engine.track_rigid).  Nothing in the reference does this:
+        its poses come from proj*.txt.  Volumes are passed as to fuseDepths with the same scale and center: numpy volumes are
+        uploaded, CUDA tensors are read in place, None tracks against the object's resident volume (the one compute_live_tsdf
+        fills; pass the scale and center it fused with).  A sharded (slab) volume is refused.  delta: Huber threshold (world
+        units), default 0.5 tdist.  Raises ValueError when fewer than `min_pixels` pixels meet the fused surface.  Returns
+        engine.TrackResult (lw, cost, pixels, iterations, converged, residual); want_residual=True adds the finest level's
+        residual map (CUDA float64 (ceil(rows/s), ceil(cols/s)) for the last stride s: the signed distance of each pixel to the
+        model, NaN where it did not contribute).  Intended loop: `lw = fus.track(dm, lw, T, W, s, c).lw;
+        fus.fuseDepths(dm, lw, T, W, s, c)`."""
+        if tsdf is None:
+            if self._vol is None:
+                raise ValueError('the volume has not been initialised')
+            vol = self._vol
+        else:
+            if tsdf.ndim != 3:
+                raise ValueError('Only 3D numpy array is accepted as tsdf')
+            if isinstance(tsdf, torch.Tensor) and tsdf.is_cuda:
+                vol = (tsdf, tsdf_w)
+            else:
+                vol = (engine._to_dev(tsdf, torch.float32, self._device), engine._to_dev(tsdf_w, torch.float32, self._device))
+        d = engine._to_dev(dm, torch.float32, self._device)
+        if d.dim() != 2:
+            raise ValueError('depth map must be 2-D')
+        delta = 0.5 * self._tdist if delta is None else float(delta)
+
+        def normal_eq(pose, stride, want=False):
+            return engine.track_normal_eq(vol, self._tsdf_res, d, pose, self._K, self._Kinv, scale, center, stride, self._tdist,
+                                          delta, want_residual=want)
+
+        res = engine.track_rigid(normal_eq, lw, strides, iterations, min_pixels=min_pixels, scale=scale)
+        if want_residual:
+            res = res._replace(residual=normal_eq(res.lw, strides[-1], True)[1])
+        return res
+
     def marching_cubes(self, tsdf=None, step_size=1):
         """core/fusion_dm.py:319-331: same as Fusion.marching_cubes but the step size defaults to 1 (the reference's FusionDM also
         leaves skimage's allow_degenerate at its default True here; the device extractor always drops degenerate triangles)."""

@@ -265,6 +265,24 @@ int dfb_corr_projective(const double* warped_pts, const double* warped_normals, 
 int64_t dfb_render_workspace_words(int64_t n_faces, int n_views, int rows, int cols);
 int dfb_render(const double* pts, int64_t n_pts, const int32_t* faces, int64_t n_faces, const dfb_views* views,
                uint64_t* workspace, int64_t workspace_words, float* depth, int32_t* face, float* normal, dfb_stream_t stream);
+/* Rigid tracking of a depth frame against the whole fused FusionDM volume (nothing in the reference: compute_live_tsdf's
+ * useICP branch, core/fusion_dm.py, needs a pose file).  Every pixel (r, c) with r % stride == 0 and c % stride == 0 and depth
+ * z = -depth[r][c] > 0 is back-projected, x = Kinv [c z, r z, z], and moved to the world by the pose lw34 = [R|t]
+ * (world -> camera, as in dfb_fuse_depth_rigid): p = R^T (x - t), grid coordinate g = (p - center) / scale + tsdf_res / 2.
+ * It contributes when the 8 corners of its trilinear cell (0 <= floor(g) <= r - 2 on every axis) all have weight > 0 and
+ * |tsdf| * scale < tdist.  Its residual is rho = scale * D, D the standard trilinear interpolant of the cell (along z, then y,
+ * then x; not the swapped weights of interpolate_tsdf), its Jacobian J = [grad D, p x grad D] for the twist (tau, omega) acting
+ * on world points as p + tau + omega x p, its Huber weight w = min(1, delta / |rho|) (oracle/track.py).
+ * out29 (device): upper triangle of H = sum w J^T J (21, row-major), g = sum w J rho (6), the Huber cost, the pixel count.
+ * residual (device, optional): [ceil(rows/stride)][ceil(cols/stride)] rho of every sampled pixel, NaN where it did not
+ * contribute.  K is the matrix Kinv inverts (checked, not read).  workspace: dfb_track_workspace_doubles(rows, cols, stride)
+ * doubles (-1 for invalid arguments).  A slab volume (x0 != 0 or x1 != rx) is refused.  No atomics: a call's sums are
+ * identical run to run. */
+int64_t dfb_track_workspace_doubles(int rows, int cols, int stride);
+int dfb_track_normal_eq(const dfb_volume* vol, int tsdf_res, double scale, const double center[3], const float* depth, int rows,
+                        int cols, const double K[9], const double Kinv[9], const double lw34[12], int stride, double tdist,
+                        double delta, double* workspace, int64_t workspace_doubles, double* out29, double* residual,
+                        dfb_stream_t stream);
 /* core/fusion.py:211-215: unsupported [m] = 1 where min over the k nearest nodes of |node - vert| / dg_w >= 1. */
 int dfb_graph_unsupported(const float* verts, int64_t m, const int32_t* vert_knn, int k, const float* node_pos,
                           const float* node_w, uint8_t* unsupported, dfb_stream_t stream);
