@@ -119,6 +119,8 @@ def declare(lib, prefix="dfb_", device=True):
         "track_workspace_doubles": ([C.c_int, C.c_int, C.c_int], C.c_int64),
         "track_normal_eq": ([C.POINTER(Volume), C.c_int, C.c_double, c_f64p, vp, C.c_int, C.c_int, c_f64p, c_f64p, c_f64p, C.c_int,
                              C.c_double, C.c_double, vp, C.c_int64, vp, vp, vp], C.c_int),
+        "raycast": ([C.POINTER(Volume), C.c_int, C.c_double, c_f64p, C.POINTER(Views), C.c_double, C.c_double, C.c_double,
+                     C.c_double, vp, vp, vp], C.c_int),
         "graph_unsupported": ([vp, C.c_int64, vp, C.c_int, vp, vp, vp, vp], C.c_int),
         "graph_sample_rounds": ([C.POINTER(PointGrid), C.c_double, C.c_int, vp, vp, vp], C.c_int),
         "mc_level_scratch_floats": ([], C.c_int64),
@@ -184,7 +186,7 @@ EXPORTS = [
     "dfb_gn_residuals", "dfb_gn_residuals_lw", "dfb_gn_pattern_rows", "dfb_gn_pattern_cols", "dfb_gn_normal_eq",
     "dfb_gn_lw_normal_eq", "dfb_gn_solve_workspace_doubles", "dfb_gn_solve",
     "dfb_point_grid_scratch_ints", "dfb_point_grid_build", "dfb_point_grid_knn", "dfb_corr_select", "dfb_corr_projective", "dfb_render_workspace_words", "dfb_render",
-    "dfb_track_workspace_doubles", "dfb_track_normal_eq", "dfb_graph_unsupported", "dfb_graph_sample_rounds",
+    "dfb_track_workspace_doubles", "dfb_track_normal_eq", "dfb_raycast", "dfb_graph_unsupported", "dfb_graph_sample_rounds",
     "dfb_mc_level_scratch_floats", "dfb_mc_level", "dfb_mc_rows", "dfb_mc_chunks", "dfb_mc_count", "dfb_mc_emit",
     "dfb_knn_brick_count", "dfb_knn_build_volume_radii", "dfb_knn_update_volume", "dfb_brick_nodes_update", "dfb_region_update",
     "dfb_comm_available", "dfb_comm_unique_id", "dfb_comm_init", "dfb_comm_destroy", "dfb_comm_rank", "dfb_comm_world",

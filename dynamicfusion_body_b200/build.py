@@ -11,7 +11,7 @@ _PKG = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(_PKG, "csrc")
 OBJ = os.path.join(CSRC, "_obj")
 OUT = os.path.join(_PKG, "libdfb_b200.so")
-SOURCES = ["common.cu", "tsdf.cu", "knn.cu", "gn.cu", "graph.cu", "mc.cu", "comm.cu", "step.cu", "render.cu", "track.cu"]
+SOURCES = ["common.cu", "tsdf.cu", "knn.cu", "gn.cu", "graph.cu", "mc.cu", "comm.cu", "step.cu", "render.cu", "track.cu", "raycast.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17", "-Xcompiler", "-fPIC"]
 
 

@@ -20,34 +20,41 @@ struct TrackParams {
     int rx, ry, rz;
 };
 
-// Steps 1-7 of oracle/track.py for pixel (r, c): returns false when the pixel does not contribute, else its residual
-// rho = scale * D (world units) and J = [grad D, p x grad D], the derivative of rho under p -> p + tau + omega x p.
-DFB_HDN bool track_pixel(const TrackParams& P, const float* tsdf, const float* weight, const float* depth, int r, int c,
-                         double* rho, double* J) {
-    const double z = -1.0 * (double)depth[(int64_t)r * P.cols + c];
-    if (!(z > 0.0)) return false;
+// Steps 2-4 of oracle/track.py for pixel (r, c) at camera depth z: camera point x = Kinv [c z, r z, z], world point
+// p = R^T (x - t) for lw = [R|t], grid coordinate g = (p - center) / scale + half, cell i = floor(g) and fraction f = g - i.
+// Returns false when the cell lies outside 0 <= i <= r - 2 on some axis.  Shared with the raycaster (dfb_raycast.h), so a
+// raycast depth back-projects exactly as the tracker back-projects it.
+DFB_HDN bool track_point_cell(const double* Kinv, const double* lw, const double* center, double scale, double half, int rx, int ry,
+                              int rz, int r, int c, double z, double* p, int* i, double* f) {
     const double a = dmul((double)c, z), b = dmul((double)r, z);
-    double x[3], e[3], p[3], g[3], f[3];
-    int i[3];
-    for (int k = 0; k < 3; ++k) x[k] = dot3_ref(P.Kinv + 3 * k, a, b, z);
-    for (int k = 0; k < 3; ++k) e[k] = dsub(x[k], P.lw[4 * k + 3]);
-    for (int k = 0; k < 3; ++k) p[k] = dadd(dadd(dmul(P.lw[k], e[0]), dmul(P.lw[4 + k], e[1])), dmul(P.lw[8 + k], e[2]));
-    const int R[3] = {P.rx, P.ry, P.rz};
+    double x[3], e[3];
+    for (int k = 0; k < 3; ++k) x[k] = dot3_ref(Kinv + 3 * k, a, b, z);
+    for (int k = 0; k < 3; ++k) e[k] = dsub(x[k], lw[4 * k + 3]);
+    for (int k = 0; k < 3; ++k) p[k] = dadd(dadd(dmul(lw[k], e[0]), dmul(lw[4 + k], e[1])), dmul(lw[8 + k], e[2]));
+    const int R[3] = {rx, ry, rz};
     for (int k = 0; k < 3; ++k) {
-        g[k] = dadd(ddiv(dsub(p[k], P.center[k]), P.scale), P.half);
-        const double fl = floor(g[k]);
+        const double g = dadd(ddiv(dsub(p[k], center[k]), scale), half);
+        const double fl = floor(g);
         if (!(fl >= 0.0 && fl <= (double)(R[k] - 2))) return false;
         i[k] = (int)fl;
-        f[k] = dsub(g[k], fl);
+        f[k] = dsub(g, fl);
     }
+    return true;
+}
+
+// Steps 5-6 for cell i at fraction f of a (rx, ry, rz) volume: false unless every one of the 8 corners has weight > 0 and
+// |tsdf| * scale < tdist (the first failing corner decides), else D, the standard trilinear interpolant (along z, then y,
+// then x), and n = grad D per grid unit.
+DFB_HDN bool track_cell_value(const float* tsdf, const float* weight, int ry, int rz, double scale, double tdist, const int* i,
+                              const double* f, double* D, double* n) {
     // corners v[dx][dy][dz]; every one observed and inside the truncation band
     double v[2][2][2];
     for (int dx = 0; dx < 2; ++dx)
         for (int dy = 0; dy < 2; ++dy)
             for (int dz = 0; dz < 2; ++dz) {
-                const int64_t o = ((int64_t)(i[0] + dx) * P.ry + (i[1] + dy)) * P.rz + (i[2] + dz);
+                const int64_t o = ((int64_t)(i[0] + dx) * ry + (i[1] + dy)) * rz + (i[2] + dz);
                 const double t = (double)tsdf[o];
-                if (!((double)weight[o] > 0.0) || !(dmul(fabs(t), P.scale) < P.tdist)) return false;
+                if (!((double)weight[o] > 0.0) || !(dmul(fabs(t), scale) < tdist)) return false;
                 v[dx][dy][dz] = t;
             }
     const double ix = dsub(1.0, f[0]), iy = dsub(1.0, f[1]), iz = dsub(1.0, f[2]);
@@ -63,8 +70,23 @@ DFB_HDN bool track_pixel(const TrackParams& P, const float* tsdf, const float* w
         gy[dx] = dsub(ez[dx][1], ez[dx][0]);
         gzy[dx] = dadd(dmul(gz[dx][0], iy), dmul(gz[dx][1], f[1]));
     }
-    const double D = dadd(dmul(ey[0], ix), dmul(ey[1], f[0]));
-    const double n[3] = {dsub(ey[1], ey[0]), dadd(dmul(gy[0], ix), dmul(gy[1], f[0])), dadd(dmul(gzy[0], ix), dmul(gzy[1], f[0]))};
+    *D = dadd(dmul(ey[0], ix), dmul(ey[1], f[0]));
+    n[0] = dsub(ey[1], ey[0]);
+    n[1] = dadd(dmul(gy[0], ix), dmul(gy[1], f[0]));
+    n[2] = dadd(dmul(gzy[0], ix), dmul(gzy[1], f[0]));
+    return true;
+}
+
+// Steps 1-7 of oracle/track.py for pixel (r, c): returns false when the pixel does not contribute, else its residual
+// rho = scale * D (world units) and J = [grad D, p x grad D], the derivative of rho under p -> p + tau + omega x p.
+DFB_HDN bool track_pixel(const TrackParams& P, const float* tsdf, const float* weight, const float* depth, int r, int c,
+                         double* rho, double* J) {
+    const double z = -1.0 * (double)depth[(int64_t)r * P.cols + c];
+    if (!(z > 0.0)) return false;
+    double p[3], f[3], n[3], D;
+    int i[3];
+    if (!track_point_cell(P.Kinv, P.lw, P.center, P.scale, P.half, P.rx, P.ry, P.rz, r, c, z, p, i, f)) return false;
+    if (!track_cell_value(tsdf, weight, P.ry, P.rz, P.scale, P.tdist, i, f, &D, n)) return false;
     *rho = dmul(P.scale, D);
     J[0] = n[0]; J[1] = n[1]; J[2] = n[2];
     J[3] = dsub(dmul(p[1], n[2]), dmul(p[2], n[1]));

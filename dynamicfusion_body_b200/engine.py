@@ -652,6 +652,38 @@ def track_rigid(normal_eq, lw0, strides=(4, 2, 1), iterations=10, lam0=1e-4, min
     return TrackResult(lw, cost / n, n, tuple(iters), converged)
 
 
+def raycast_far(shape, tsdf_res, views, scale, center):
+    """The largest camera depth (z of E [p, 1]) of the 8 corner voxels of a (rx, ry, rz) volume on the grid of `raycast`, over
+    the views (identity without extrinsics): beyond it no ray meets the volume."""
+    idx = np.stack(np.meshgrid(*[(0.0, r - 1.0) for r in shape], indexing="ij"), -1).reshape(-1, 3)
+    p = scale * (idx - tsdf_res / 2.0) + np.asarray(center, dtype=np.float64).reshape(3)
+    rows = [np.array(views.E[v][8:12]) for v in range(views.n_views)] if views.has_extrinsics else [np.array([0.0, 0.0, 1.0, 0.0])]
+    return max(float((p @ e[:3] + e[3]).max()) for e in rows)
+
+
+def raycast(vol, tsdf_res, views, scale, center, tdist, step=None, z_near=0.0, z_far=None):
+    """dfb_raycast: depth and normal maps of the whole volume `vol` (a DeviceVolume or a (tsdf, weight) pair of float32 CUDA
+    tensors, read in place) from the cameras of `camera_views` (K, image size, world -> camera extrinsics), on the grid of
+    fuseDepths (grid = (p - center) / scale + tsdf_res / 2) with the truncation distance tdist.  Each ray is sampled every `step`
+    (world units along camera z; default `scale`, one voxel) from z_near to z_far (default: the largest camera depth of the
+    volume's corner voxels, `raycast_far`) and stops at its first zero crossing of the tracker's interpolant.  Returns CUDA
+    tensors depth (V,rows,cols) float32 (negative depth, 0 = no hit: the convention of fuseDepths, track and fuseFrame) and
+    normal (V,rows,cols,3) float32 (the unit gradient of the field in the world frame, 0 = none)."""
+    v = _volume_struct(vol)
+    dev = vol.device if isinstance(vol, DeviceVolume) else vol[0].device
+    step = float(scale) if step is None else float(step)
+    center = np.ascontiguousarray(np.zeros(3) if center is None else center, dtype=np.float64).reshape(3)
+    if z_far is None:
+        # nothing of the volume in front of the cameras: one step of range, every ray misses
+        z_far = max(raycast_far((v.rx, v.ry, v.rz), tsdf_res, views, scale, center), float(z_near) + step)
+    V, rows, cols = views.n_views, views.rows, views.cols
+    depth = torch.empty((V, rows, cols), dtype=torch.float32, device=dev)
+    normal = torch.empty((V, rows, cols, 3), dtype=torch.float32, device=dev)
+    _capi.check(_capi.lib().dfb_raycast(C.byref(v), int(tsdf_res), float(scale), center.ctypes.data_as(_capi.c_f64p), C.byref(views),
+                                        float(tdist), step, float(z_near), float(z_far), _ptr(depth), _ptr(normal), _stream()))
+    return depth, normal
+
+
 def graph_unsupported(wf, verts, vert_knn):
     """core/fusion.py:211-215: bool (m,) -- surface points no node of `wf` supports."""
     dev = wf.device

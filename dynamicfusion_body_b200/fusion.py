@@ -30,6 +30,7 @@ from . import gn as _gn
 
 
 LiveRender = collections.namedtuple("LiveRender", ["depth", "normal", "face", "vertices", "faces"])
+Raycast = collections.namedtuple("Raycast", ["depth", "normal"])
 
 
 def _as_np(a):
@@ -737,6 +738,18 @@ class FusionDM(_FusionBase):
             return (tsdf, tsdf_w)
         return (out_t, out_w)
 
+    def _whole_volume(self, tsdf, tsdf_w):
+        """The volume `track` and `raycast` read: the resident one for None, CUDA tensors in place, numpy uploaded."""
+        if tsdf is None:
+            if self._vol is None:
+                raise ValueError('the volume has not been initialised')
+            return self._vol
+        if tsdf.ndim != 3:
+            raise ValueError('Only 3D numpy array is accepted as tsdf')
+        if isinstance(tsdf, torch.Tensor) and tsdf.is_cuda:
+            return (tsdf, tsdf_w)
+        return (engine._to_dev(tsdf, torch.float32, self._device), engine._to_dev(tsdf_w, torch.float32, self._device))
+
     def track(self, dm, lw, tsdf=None, tsdf_w=None, scale=1.0, center=np.zeros(3), *, strides=(4, 2, 1), iterations=10, delta=None,
               min_pixels=100, want_residual=False):
         """The camera pose of the depth frame `dm` (negative depth, 0 = no data) against the fused volume, from the initial pose
@@ -750,17 +763,7 @@ class FusionDM(_FusionBase):
         residual map (CUDA float64 (ceil(rows/s), ceil(cols/s)) for the last stride s: the signed distance of each pixel to the
         model, NaN where it did not contribute).  Intended loop: `lw = fus.track(dm, lw, T, W, s, c).lw;
         fus.fuseDepths(dm, lw, T, W, s, c)`."""
-        if tsdf is None:
-            if self._vol is None:
-                raise ValueError('the volume has not been initialised')
-            vol = self._vol
-        else:
-            if tsdf.ndim != 3:
-                raise ValueError('Only 3D numpy array is accepted as tsdf')
-            if isinstance(tsdf, torch.Tensor) and tsdf.is_cuda:
-                vol = (tsdf, tsdf_w)
-            else:
-                vol = (engine._to_dev(tsdf, torch.float32, self._device), engine._to_dev(tsdf_w, torch.float32, self._device))
+        vol = self._whole_volume(tsdf, tsdf_w)
         d = engine._to_dev(dm, torch.float32, self._device)
         if d.dim() != 2:
             raise ValueError('depth map must be 2-D')
@@ -774,6 +777,29 @@ class FusionDM(_FusionBase):
         if want_residual:
             res = res._replace(residual=normal_eq(res.lw, strides[-1], True)[1])
         return res
+
+    def raycast(self, lw, tsdf=None, tsdf_w=None, scale=1.0, center=np.zeros(3), *, rows=480, cols=640, K=None, step=None, z_near=0.0,
+                z_far=None):
+        """Depth and normal maps of the fused volume seen from the pose `lw` (one 3x4 world -> camera, the `lw` of fuseDepths and
+        track, or a (V,3,4) stack of at most 8), raycast on the device (include/dfb.h dfb_raycast) with no surface extraction:
+        the model's view from a tracked pose, to compare with the input frame.  Nothing in the reference does this.  Volumes are
+        passed as to track, with the scale and center they were fused with: numpy volumes are uploaded, CUDA tensors are read in
+        place, None reads the object's resident volume; a sharded (slab) volume is refused.  K defaults to the object's.  Each
+        ray is sampled every `step` (world units along camera z, default one voxel, `scale`) from z_near to z_far (default: the
+        farthest corner of the volume) and stops at its first zero crossing of the tracker's interpolant.  Returns
+        Raycast(depth (V,rows,cols) float32, negative depth, 0 = no surface, the convention fuseDepths, track and fuseFrame take;
+        normal (V,rows,cols,3) float32, the field's unit gradient in the world frame, 0 = none) as CUDA tensors.  Intended loop:
+        `lw = fus.track(dm, lw, T, W, s, c).lw; fus.fuseDepths(dm, lw, T, W, s, c); model = fus.raycast(lw, T, W, s, c)`."""
+        E = np.asarray(lw, dtype=np.float64)
+        if E.shape == (3, 4):
+            E = E[None]
+        if E.ndim != 3 or E.shape[1:] != (3, 4):
+            raise ValueError('lw must be a 3x4 pose or a (views, 3, 4) stack')
+        K = self._K if K is None else np.asarray(K, dtype=np.float64)
+        vol = self._whole_volume(tsdf, tsdf_w)
+        views = engine.camera_views(K, rows, cols, E)
+        depth, normal = engine.raycast(vol, self._tsdf_res, views, scale, center, self._tdist, step, z_near, z_far)
+        return Raycast(depth, normal)
 
     def marching_cubes(self, tsdf=None, step_size=1):
         """core/fusion_dm.py:319-331: same as Fusion.marching_cubes but the step size defaults to 1 (the reference's FusionDM also

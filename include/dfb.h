@@ -283,6 +283,19 @@ int dfb_track_normal_eq(const dfb_volume* vol, int tsdf_res, double scale, const
                         int cols, const double K[9], const double Kinv[9], const double lw34[12], int stride, double tdist,
                         double delta, double* workspace, int64_t workspace_doubles, double* out29, double* residual,
                         dfb_stream_t stream);
+/* Raycasting of the whole fused FusionDM volume (nothing in the reference, which can only extract the surface): depth and
+ * normal maps of the model from every view of `views` (K is not read, Kinv is; E[v] = [R|t] world -> camera as in
+ * dfb_fuse_depth_rigid, identity without extrinsics; depth pointers ignored).  Pixel (r, c) of view v samples its ray at
+ * z_k = z_near + k step (camera z, world units) while z_k <= z_far, each sample back-projected and gated exactly as
+ * dfb_track_normal_eq back-projects and gates a pixel of depth z_k (grid g = (p - center) / scale + tsdf_res / 2, all 8
+ * corners observed with |tsdf| * scale < tdist, standard trilinear D).  The first pair of consecutive valid samples with
+ * D_k > 0 >= D_k+1 is a hit, refined once, z* = z_k + step D_k / (D_k - D_k+1); D_k < 0 <= D_k+1 (a back face) ends the ray
+ * with no hit.  depth [V][rows][cols] (device): -float(z*), 0 = no hit; normal [V][rows][cols][3] (device): grad D / |grad D| at
+ * z* in the world frame, 0 = no hit or zero gradient.  The march is clipped to the volume's box (oracle/raycast.py).
+ * A slab volume (x0 != 0 or x1 != rx) is refused.  Needs step > 0, 0 <= z_near < z_far (finite), (z_far - z_near) / step < 2^30.
+ * One thread per ray, no atomics: identical run to run. */
+int dfb_raycast(const dfb_volume* vol, int tsdf_res, double scale, const double center[3], const dfb_views* views, double tdist,
+                double step, double z_near, double z_far, float* depth, float* normal, dfb_stream_t stream);
 /* core/fusion.py:211-215: unsupported [m] = 1 where min over the k nearest nodes of |node - vert| / dg_w >= 1. */
 int dfb_graph_unsupported(const float* verts, int64_t m, const int32_t* vert_knn, int k, const float* node_pos,
                           const float* node_w, uint8_t* unsupported, dfb_stream_t stream);
