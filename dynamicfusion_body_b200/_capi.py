@@ -76,13 +76,13 @@ class PointGrid(C.Structure):
                 ("dims", C.c_int * 3), ("cell_start", C.c_void_p), ("order", C.c_void_p)]
 
 
-def declare(lib, prefix="dfb_", device=True):
+def declare(lib):
     """Attach argtypes/restype for every entry point of include/dfb.h present in `lib`."""
     vp = C.c_void_p
     sig = {
         "version": ([], C.c_int),
         "last_error": ([], C.c_char_p),
-        "nodes_pack": ([vp, vp, vp, C.c_int, vp] + ([vp] if device else []), None if not device else C.c_int),
+        "nodes_pack": ([vp, vp, vp, C.c_int, vp, vp], C.c_int),
         "knn_build_volume": ([vp, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, vp, vp], C.c_int),
         "knn_brick_count": ([C.c_int, C.c_int, C.c_int], C.c_int64),
         "knn_build_volume_radii": ([vp, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, vp, vp, vp], C.c_int),
@@ -100,22 +100,22 @@ def declare(lib, prefix="dfb_", device=True):
                               c_f64p, C.c_double, C.c_double, C.c_int, C.POINTER(Workspace), vp, vp, vp], C.c_int),
         "tsdf_update_volume": ([C.POINTER(Volume), C.POINTER(WarpField), vp, C.c_int, C.c_int, C.c_int, C.c_double,
                                 C.c_double, C.c_int, C.POINTER(Workspace), vp, vp], C.c_int),
-        "warp_points": ([vp, vp, C.c_int64, vp, C.POINTER(WarpField), vp, vp] + ([vp] if device else []), C.c_int),
-        "dq_blend_points": ([vp, C.c_int64, vp, C.POINTER(WarpField), vp] + ([vp] if device else []), C.c_int),
-        "gn_residuals": ([C.POINTER(GNProblem), vp, C.c_int, vp] + ([vp] if device else []), C.c_int),
-        "gn_residuals_lw": ([C.POINTER(GNProblem), vp, C.c_int, c_f64p, C.c_int, vp] + ([vp] if device else []), C.c_int),
+        "warp_points": ([vp, vp, C.c_int64, vp, C.POINTER(WarpField), vp, vp, vp], C.c_int),
+        "dq_blend_points": ([vp, C.c_int64, vp, C.POINTER(WarpField), vp, vp], C.c_int),
+        "gn_residuals": ([C.POINTER(GNProblem), vp, C.c_int, vp, vp], C.c_int),
+        "gn_residuals_lw": ([C.POINTER(GNProblem), vp, C.c_int, c_f64p, C.c_int, vp, vp], C.c_int),
         "gn_pattern_rows": ([C.POINTER(GNProblem), vp, vp, vp], C.c_int),
         "gn_pattern_cols": ([C.c_int, vp, vp, vp, vp], C.c_int),
-        "gn_normal_eq": ([C.POINTER(GNProblem), vp, vp, vp, C.c_int64, vp, vp, vp] + ([vp] if device else []), C.c_int),
-        "gn_lw_normal_eq": ([C.POINTER(GNProblem), vp, c_f64p, vp, vp, vp] + ([vp] if device else []), C.c_int),
+        "gn_normal_eq": ([C.POINTER(GNProblem), vp, vp, vp, C.c_int64, vp, vp, vp, vp], C.c_int),
+        "gn_lw_normal_eq": ([C.POINTER(GNProblem), vp, c_f64p, vp, vp, vp, vp], C.c_int),
         "gn_solve_workspace_doubles": ([C.c_int], C.c_int64),
         "point_grid_scratch_ints": ([C.c_int64], C.c_int64),
         "point_grid_build": ([C.POINTER(PointGrid), vp, vp, vp, vp], C.c_int),
         "point_grid_knn": ([C.POINTER(PointGrid), vp, C.c_int64, C.c_int, vp, vp, vp], C.c_int),
         "corr_select": ([vp, vp, C.c_int64, vp, vp, C.c_int, vp, vp, vp], C.c_int),
-        "corr_projective": ([vp, vp, C.c_int64, C.POINTER(Views), C.c_double, C.c_double, vp, vp, vp] + ([vp] if device else []), C.c_int),
+        "corr_projective": ([vp, vp, C.c_int64, C.POINTER(Views), C.c_double, C.c_double, vp, vp, vp, vp], C.c_int),
         "render_workspace_words": ([C.c_int64, C.c_int, C.c_int, C.c_int], C.c_int64),
-        "render": ([vp, C.c_int64, vp, C.c_int64, C.POINTER(Views), vp, C.c_int64, vp, vp, vp] + ([vp] if device else []), C.c_int),
+        "render": ([vp, C.c_int64, vp, C.c_int64, C.POINTER(Views), vp, C.c_int64, vp, vp, vp, vp], C.c_int),
         "track_workspace_doubles": ([C.c_int, C.c_int, C.c_int], C.c_int64),
         "track_normal_eq": ([C.POINTER(Volume), C.c_int, C.c_double, c_f64p, vp, C.c_int, C.c_int, c_f64p, c_f64p, c_f64p, C.c_int,
                              C.c_double, C.c_double, vp, C.c_int64, vp, vp, vp], C.c_int),
@@ -147,7 +147,7 @@ def declare(lib, prefix="dfb_", device=True):
         "frame_step_stats": ([vp, C.POINTER(C.c_int64)], C.c_int),
     }
     for name, (argtypes, restype) in sig.items():
-        fn = getattr(lib, prefix + name, None)
+        fn = getattr(lib, "dfb_" + name, None)
         if fn is None:
             continue
         fn.argtypes = argtypes

@@ -4,22 +4,11 @@
 #include <stdarg.h>
 #include <stdio.h>
 
-#include "../../include/dfb.h"
+#include "dfb_require.h"
 
 namespace dfb {
-void set_error(const char* fmt, ...);
 int check_cuda(cudaError_t e, const char* what);
 }  // namespace dfb
-
-#ifndef DFB_REQUIRE
-#define DFB_REQUIRE(cond, ...)            \
-    do {                                  \
-        if (!(cond)) {                    \
-            dfb::set_error(__VA_ARGS__);  \
-            return DFB_ERR_INVALID;       \
-        }                                 \
-    } while (0)
-#endif
 
 #define DFB_CUDA(call)                                   \
     do {                                                 \

@@ -14,6 +14,8 @@
 #include <math.h>
 #include <stdint.h>
 
+#include "dfb_require.h"
+
 #if defined(__CUDACC__)
 #define DFB_HD __host__ __device__ __forceinline__
 #define DFB_HDN inline __host__ __device__
@@ -412,6 +414,19 @@ DFB_HDN int assoc_projective_ref(const double* w, const double* m, const float* 
     *cost_out = best_cost;
     corr_out[0] = bc[0]; corr_out[1] = bc[1]; corr_out[2] = bc[2];
     return best;
+}
+
+// The checks of dfb_corr_projective; its kernel reads `views` as it stands.
+inline int check_corr_projective(const double* warped_pts, const double* warped_normals, int64_t m, const dfb_views* views,
+                                 double max_distance, double min_normal_dot, const int32_t* view, const double* cost,
+                                 const double* corr) {
+    DFB_REQUIRE(warped_pts && warped_normals && views && view && cost && corr && m >= 0, "null pointer / negative count");
+    DFB_REQUIRE(views->n_views >= 1 && views->n_views <= DFB_MAX_VIEWS, "n_views=%d out of range [1,%d]", views->n_views, DFB_MAX_VIEWS);
+    DFB_REQUIRE(views->rows >= 3 && views->cols >= 3, "depth map %dx%d smaller than 3x3", views->rows, views->cols);
+    for (int v = 0; v < views->n_views; ++v) DFB_REQUIRE(views->depth[v], "depth[%d] is null", v);
+    DFB_REQUIRE(max_distance > 0, "max_distance must be positive");
+    DFB_REQUIRE(min_normal_dot >= -1.0 && min_normal_dot <= 1.0, "min_normal_dot must be in [-1,1]");
+    return DFB_OK;
 }
 
 // core/util.py:102-137 interpolate_tsdf on a float32 live volume; returns false for "None".

@@ -7,20 +7,10 @@
 #include <stdio.h>
 #include <string.h>
 
-#include "../../include/dfb.h"
+#include "dfb_require.h"
 #include "dfb_voxel.h"
 
 namespace dfb {
-
-void set_error(const char* fmt, ...);  // provided by common.cu (library) or the test shim
-
-#define DFB_REQUIRE(cond, ...)            \
-    do {                                  \
-        if (!(cond)) {                    \
-            dfb::set_error(__VA_ARGS__);  \
-            return DFB_ERR_INVALID;       \
-        }                                 \
-    } while (0)
 
 inline void mat34_mul(const double* A, const double* B, double* C) {  // C = A * B as 4x4 affine maps
     for (int r = 0; r < 3; ++r)

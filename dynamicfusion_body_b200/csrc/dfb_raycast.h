@@ -3,8 +3,9 @@
 // The definition is oracle/raycast.py.  Every sample goes through the tracker's own functions (dfb_track.h: track_point_cell,
 // track_cell_value), so the raycast surface is the one dfb_track_normal_eq aligns frames to, and every float64 operation of the
 // march, the refinement and the box clip is written in the oracle's order with the explicit-rounding helpers of dfb_math.h:
-// the device kernel and the test suite's host build (tests/raycast_shim.py) both reproduce every ray bit for bit.
+// the device kernel and the test suite's host build both reproduce every ray bit for bit.
 #pragma once
+#include "dfb_require.h"
 #include "dfb_track.h"
 
 namespace dfb {
@@ -16,6 +17,40 @@ struct RaycastParams {
     double scale, half, tdist, step, z_near, z_far;
     int rows, cols, rx, ry, rz;
 };
+
+// The cameras: the inverse intrinsics and one world -> camera pose per view (the identity without extrinsics).
+struct RaycastCams {
+    double Kinv[9];
+    double E[DFB_MAX_VIEWS * 12];
+};
+
+// The checks of dfb_raycast, and the blocks of the call.
+inline int build_raycast(RaycastParams& P, RaycastCams& cams, const dfb_volume* vol, int tsdf_res, double scale, const double* center,
+                         const dfb_views* views, double tdist, double step, double z_near, double z_far, const float* depth,
+                         const float* normal) {
+    DFB_REQUIRE(vol && center && views && depth && normal, "null pointer");
+    DFB_REQUIRE(vol->tsdf && vol->weight, "null pointer (volume)");
+    DFB_REQUIRE(vol->rx >= 2 && vol->ry >= 2 && vol->rz >= 2, "volume %dx%dx%d is smaller than one cell", vol->rx, vol->ry, vol->rz);
+    DFB_REQUIRE(vol->x0 == 0 && vol->x1 == vol->rx, "slab [%d,%d) of %d planes: raycasting needs the whole volume (trilinear cells "
+                "span neighbouring planes)", vol->x0, vol->x1, vol->rx);
+    DFB_REQUIRE(tsdf_res >= 1, "tsdf_res=%d must be positive", tsdf_res);
+    DFB_REQUIRE(views->n_views >= 1 && views->n_views <= DFB_MAX_VIEWS, "n_views=%d out of range [1,%d]", views->n_views, DFB_MAX_VIEWS);
+    DFB_REQUIRE(views->rows >= 1 && views->cols >= 1, "image %dx%d is empty", views->rows, views->cols);
+    DFB_REQUIRE(scale > 0, "scale must be positive");
+    DFB_REQUIRE(tdist > 0, "truncation distance must be positive");
+    DFB_REQUIRE(step > 0, "ray step must be positive");
+    DFB_REQUIRE(isfinite(z_near) && isfinite(z_far) && z_near >= 0 && z_near < z_far, "ray range z_near=%g, z_far=%g: need "
+                "0 <= z_near < z_far, both finite", z_near, z_far);
+    DFB_REQUIRE((z_far - z_near) / step < 1073741824.0, "ray range of (z_far - z_near) / step = %g samples exceeds 2^30",
+                (z_far - z_near) / step);
+    for (int i = 0; i < 3; ++i) P.center[i] = center[i];
+    P.scale = scale; P.half = tsdf_res / 2.0; P.tdist = tdist; P.step = step; P.z_near = z_near; P.z_far = z_far;
+    P.rows = views->rows; P.cols = views->cols; P.rx = vol->rx; P.ry = vol->ry; P.rz = vol->rz;
+    for (int i = 0; i < 9; ++i) cams.Kinv[i] = views->Kinv[i];
+    for (int v = 0; v < views->n_views; ++v)
+        for (int i = 0; i < 12; ++i) cams.E[12 * v + i] = views->has_extrinsics ? views->E[v][i] : (i % 5 == 0 ? 1.0 : 0.0);
+    return DFB_OK;
+}
 
 // Step 5 of oracle/raycast.py: the range [*k0, *k1] of samples the ray of pixel (r, c) can take (*k0 > *k1: none).  The ray's
 // grid coordinate og + z dg is clipped to the box [-1/2, r_a - 1/2] (half a cell wider than the cell range) and the range is

@@ -1,13 +1,14 @@
 // dfb_render.h -- per-face and per-pixel arithmetic of the z-buffer rasteriser (csrc/render.cu, include/dfb.h dfb_render).
 //
 // The definition is oracle/render.py; every float64 operation below is written in its order with the explicit-rounding
-// helpers of dfb_math.h, so the device kernels and the test suite's host build (tests/render_shim.py) both reproduce it bit for
-// bit.  The winner of a pixel is the smallest 64-bit key (float32 depth bits << 32 | face id): an atomicMin on the device, a
-// plain min on the host, and the result does not depend on the order in which faces arrive.
+// helpers of dfb_math.h, so the device kernels and the test suite's host build both reproduce it bit for bit.
+// The winner of a pixel is the smallest 64-bit key (float32 depth bits << 32 | face id): an atomicMin on the device, a plain
+// min on the host, and the result does not depend on the order in which faces arrive.
 #pragma once
 #include <string.h>
 
 #include "dfb_math.h"
+#include "dfb_require.h"
 
 namespace dfb {
 
@@ -21,6 +22,28 @@ struct RenderFace {
     double A;
     int c0, c1, r0, r1;
 };
+
+// The cameras of one call: intrinsics, one world -> camera extrinsic per view when has_e, and the image size.
+struct RenderCams {
+    double K[9];
+    double E[DFB_MAX_VIEWS * 12];
+    int n_views, rows, cols, has_e;
+};
+
+// The checks of dfb_render other than its workspace's, and the camera block of the call.
+inline int build_render(RenderCams& cams, const double* pts, int64_t n_pts, const int32_t* faces, int64_t n_faces, const dfb_views* views,
+                        const float* depth, const int32_t* face, const float* normal) {
+    DFB_REQUIRE(views && depth && face && normal && (pts || n_pts == 0) && (faces || n_faces == 0), "null pointer");
+    DFB_REQUIRE(n_pts >= 0 && n_faces >= 0, "negative count");
+    DFB_REQUIRE(n_faces <= INT32_MAX, "n_faces=%lld exceeds the int32 face ids", (long long)n_faces);
+    DFB_REQUIRE(views->n_views >= 1 && views->n_views <= DFB_MAX_VIEWS, "n_views=%d out of range [1,%d]", views->n_views, DFB_MAX_VIEWS);
+    DFB_REQUIRE(views->rows >= 1 && views->cols >= 1, "image %dx%d is empty", views->rows, views->cols);
+    for (int i = 0; i < 9; ++i) cams.K[i] = views->K[i];
+    for (int v = 0; v < views->n_views; ++v)
+        for (int i = 0; i < 12; ++i) cams.E[12 * v + i] = views->E[v][i];
+    cams.n_views = views->n_views; cams.rows = views->rows; cams.cols = views->cols; cams.has_e = views->has_extrinsics ? 1 : 0;
+    return DFB_OK;
+}
 
 // E(a, b, p) = (xb - xa)(py - ya) - (yb - ya)(px - xa), each product rounded
 DFB_HD double render_edge(double xa, double ya, double xb, double yb, double px, double py) {

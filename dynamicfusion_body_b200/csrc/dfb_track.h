@@ -1,10 +1,11 @@
 // dfb_track.h -- per-pixel arithmetic of rigid point-to-TSDF tracking (csrc/track.cu, include/dfb.h dfb_track_normal_eq).
 //
 // The definition is oracle/track.py; every float64 operation below is written in its order with the explicit-rounding helpers
-// of dfb_math.h, so the device kernel and the test suite's host build (tests/track_shim.py) both reproduce the gate, the
-// residual and the Jacobian of every pixel bit for bit.  Only the sums over pixels differ in their order of addition.
+// of dfb_math.h, so the device kernel and the test suite's host build both reproduce the gate, the residual and the Jacobian
+// of every pixel bit for bit.  Only the sums over pixels differ in their order of addition.
 #pragma once
 #include "dfb_math.h"
+#include "dfb_require.h"
 
 namespace dfb {
 
@@ -19,6 +20,31 @@ struct TrackParams {
     int rows, cols, stride, rows_s, cols_s;   // rows_s x cols_s sampled pixels (r, c) = (stride * i, stride * j)
     int rx, ry, rz;
 };
+
+// The checks of dfb_track_normal_eq other than its workspace's, and the block of the call.
+inline int build_track(TrackParams& P, const dfb_volume* vol, int tsdf_res, double scale, const double* center, const float* depth,
+                       int rows, int cols, const double* K, const double* Kinv, const double* lw34, int stride, double tdist,
+                       double delta, const double* out29) {
+    DFB_REQUIRE(vol && center && depth && K && Kinv && lw34 && out29, "null pointer");
+    DFB_REQUIRE(vol->tsdf && vol->weight, "null pointer (volume)");
+    DFB_REQUIRE(vol->rx >= 2 && vol->ry >= 2 && vol->rz >= 2, "volume %dx%dx%d is smaller than one cell", vol->rx, vol->ry, vol->rz);
+    DFB_REQUIRE(vol->x0 == 0 && vol->x1 == vol->rx, "slab [%d,%d) of %d planes: tracking needs the whole volume (trilinear cells "
+                "span neighbouring planes)", vol->x0, vol->x1, vol->rx);
+    DFB_REQUIRE(tsdf_res >= 1, "tsdf_res=%d must be positive", tsdf_res);
+    DFB_REQUIRE(rows >= 1 && cols >= 1, "depth map %dx%d is empty", rows, cols);
+    DFB_REQUIRE(stride >= 1, "stride=%d must be >= 1", stride);
+    DFB_REQUIRE(scale > 0, "scale must be positive");
+    DFB_REQUIRE(tdist > 0, "truncation distance must be positive");
+    DFB_REQUIRE(delta > 0, "Huber threshold must be positive");
+    for (int i = 0; i < 9; ++i) P.Kinv[i] = Kinv[i];
+    for (int i = 0; i < 12; ++i) P.lw[i] = lw34[i];
+    for (int i = 0; i < 3; ++i) P.center[i] = center[i];
+    P.scale = scale; P.half = tsdf_res / 2.0; P.tdist = tdist; P.delta = delta;
+    P.rows = rows; P.cols = cols; P.stride = stride;
+    P.rows_s = (rows + stride - 1) / stride; P.cols_s = (cols + stride - 1) / stride;
+    P.rx = vol->rx; P.ry = vol->ry; P.rz = vol->rz;
+    return DFB_OK;
+}
 
 // Steps 2-4 of oracle/track.py for pixel (r, c) at camera depth z: camera point x = Kinv [c z, r z, z], world point
 // p = R^T (x - t) for lw = [R|t], grid coordinate g = (p - center) / scale + half, cell i = floor(g) and fraction f = g - i.

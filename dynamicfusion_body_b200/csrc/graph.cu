@@ -392,12 +392,7 @@ extern "C" int dfb_corr_select(const double* warped_pts, const double* warped_no
 extern "C" int dfb_corr_projective(const double* warped_pts, const double* warped_normals, int64_t m, const dfb_views* views,
                                    double max_distance, double min_normal_dot, int32_t* view, double* cost, double* corr,
                                    dfb_stream_t stream) {
-    DFB_REQUIRE(warped_pts && warped_normals && views && view && cost && corr && m >= 0, "null pointer / negative count");
-    DFB_REQUIRE(views->n_views >= 1 && views->n_views <= DFB_MAX_VIEWS, "n_views=%d out of range [1,%d]", views->n_views, DFB_MAX_VIEWS);
-    DFB_REQUIRE(views->rows >= 3 && views->cols >= 3, "depth map %dx%d smaller than 3x3", views->rows, views->cols);
-    for (int v = 0; v < views->n_views; ++v) DFB_REQUIRE(views->depth[v], "depth[%d] is null", v);
-    DFB_REQUIRE(max_distance > 0, "max_distance must be positive");
-    DFB_REQUIRE(min_normal_dot >= -1.0 && min_normal_dot <= 1.0, "min_normal_dot must be in [-1,1]");
+    if (int r = check_corr_projective(warped_pts, warped_normals, m, views, max_distance, min_normal_dot, view, cost, corr)) return r;
     if (m == 0) return DFB_OK;
     const int64_t need = (m + 127) / 128;
     const unsigned blocks = (unsigned)(need < 148 * 16 ? need : 148 * 16);   // 16 blocks per SM, grid-stride beyond

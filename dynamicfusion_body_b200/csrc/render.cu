@@ -20,22 +20,16 @@ constexpr int RENDER_SMALL_PIXELS = 16;
 constexpr int RENDER_THREADS = 256;
 constexpr int RENDER_MAX_BLOCKS = 148 * 8;   // 8 blocks per SM, grid-stride beyond
 
-struct Cams {
-    double K[9];
-    double E[DFB_MAX_VIEWS * 12];
-    int n_views, rows, cols, has_e;
-};
-
 // the camera block is read through pointers by the per-face function: staged in shared memory (indexing the kernel
 // parameter through a pointer would make every thread copy the whole struct to its local stack)
-__device__ __forceinline__ void stage_cams(const Cams& c, double* sK, double* sE) {
+__device__ __forceinline__ void stage_cams(const RenderCams& c, double* sK, double* sE) {
     for (int i = threadIdx.x; i < 9; i += blockDim.x) sK[i] = c.K[i];
     for (int i = threadIdx.x; i < 12 * c.n_views; i += blockDim.x) sE[i] = c.E[i];
     __syncthreads();
 }
 
 __global__ void __launch_bounds__(RENDER_THREADS) raster_small_kernel(const double* __restrict__ pts, int64_t n_pts,
-                                                                      const int32_t* __restrict__ faces, int64_t n_faces, const Cams cams,
+                                                                      const int32_t* __restrict__ faces, int64_t n_faces, const RenderCams cams,
                                                                       unsigned long long* __restrict__ zbuf, unsigned long long* __restrict__ n_large,
                                                                       unsigned long long* __restrict__ large) {
     __shared__ double sK[9], sE[DFB_MAX_VIEWS * 12];
@@ -76,7 +70,7 @@ __global__ void __launch_bounds__(RENDER_THREADS) raster_small_kernel(const doub
 }
 
 __global__ void __launch_bounds__(RENDER_THREADS) raster_large_kernel(const double* __restrict__ pts, int64_t n_pts,
-                                                                      const int32_t* __restrict__ faces, const Cams cams,
+                                                                      const int32_t* __restrict__ faces, const RenderCams cams,
                                                                       unsigned long long* __restrict__ zbuf, const unsigned long long* __restrict__ n_large,
                                                                       const unsigned long long* __restrict__ large) {
     __shared__ double sK[9], sE[DFB_MAX_VIEWS * 12];
@@ -128,19 +122,12 @@ extern "C" int64_t dfb_render_workspace_words(int64_t n_faces, int n_views, int 
 extern "C" int dfb_render(const double* pts, int64_t n_pts, const int32_t* faces, int64_t n_faces, const dfb_views* views,
                           uint64_t* workspace, int64_t workspace_words, float* depth, int32_t* face, float* normal,
                           dfb_stream_t stream) {
-    DFB_REQUIRE(views && workspace && depth && face && normal && (pts || n_pts == 0) && (faces || n_faces == 0), "null pointer");
-    DFB_REQUIRE(n_pts >= 0 && n_faces >= 0, "negative count");
-    DFB_REQUIRE(n_faces <= INT32_MAX, "n_faces=%lld exceeds the int32 face ids", (long long)n_faces);
-    DFB_REQUIRE(views->n_views >= 1 && views->n_views <= DFB_MAX_VIEWS, "n_views=%d out of range [1,%d]", views->n_views, DFB_MAX_VIEWS);
-    DFB_REQUIRE(views->rows >= 1 && views->cols >= 1, "image %dx%d is empty", views->rows, views->cols);
+    DFB_REQUIRE(workspace, "null pointer");
+    RenderCams cams;
+    if (int r = build_render(cams, pts, n_pts, faces, n_faces, views, depth, face, normal)) return r;
     const int64_t need = dfb_render_workspace_words(n_faces, views->n_views, views->rows, views->cols);
     DFB_REQUIRE(workspace_words >= need, "workspace of %lld words is smaller than the %lld dfb_render_workspace_words asks for",
                 (long long)workspace_words, (long long)need);
-    Cams cams;
-    for (int i = 0; i < 9; ++i) cams.K[i] = views->K[i];
-    for (int v = 0; v < views->n_views; ++v)
-        for (int i = 0; i < 12; ++i) cams.E[12 * v + i] = views->E[v][i];
-    cams.n_views = views->n_views; cams.rows = views->rows; cams.cols = views->cols; cams.has_e = views->has_extrinsics ? 1 : 0;
     const cudaStream_t s = (cudaStream_t)stream;
     const int64_t npix = (int64_t)views->n_views * views->rows * views->cols;
     unsigned long long* n_large = (unsigned long long*)workspace;

@@ -90,28 +90,12 @@ extern "C" int dfb_track_normal_eq(const dfb_volume* vol, int tsdf_res, double s
                                    int rows, int cols, const double K[9], const double Kinv[9], const double lw34[12], int stride,
                                    double tdist, double delta, double* workspace, int64_t workspace_doubles, double* out29,
                                    double* residual, dfb_stream_t stream) {
-    DFB_REQUIRE(vol && center && depth && K && Kinv && lw34 && workspace && out29, "null pointer");
-    DFB_REQUIRE(vol->tsdf && vol->weight, "null pointer (volume)");
-    DFB_REQUIRE(vol->rx >= 2 && vol->ry >= 2 && vol->rz >= 2, "volume %dx%dx%d is smaller than one cell", vol->rx, vol->ry, vol->rz);
-    DFB_REQUIRE(vol->x0 == 0 && vol->x1 == vol->rx, "slab [%d,%d) of %d planes: tracking needs the whole volume (trilinear cells "
-                "span neighbouring planes)", vol->x0, vol->x1, vol->rx);
-    DFB_REQUIRE(tsdf_res >= 1, "tsdf_res=%d must be positive", tsdf_res);
-    DFB_REQUIRE(rows >= 1 && cols >= 1, "depth map %dx%d is empty", rows, cols);
-    DFB_REQUIRE(stride >= 1, "stride=%d must be >= 1", stride);
-    DFB_REQUIRE(scale > 0, "scale must be positive");
-    DFB_REQUIRE(tdist > 0, "truncation distance must be positive");
-    DFB_REQUIRE(delta > 0, "Huber threshold must be positive");
+    DFB_REQUIRE(workspace, "null pointer");
+    TrackParams P;
+    if (int r = build_track(P, vol, tsdf_res, scale, center, depth, rows, cols, K, Kinv, lw34, stride, tdist, delta, out29)) return r;
     const int64_t need = dfb_track_workspace_doubles(rows, cols, stride);
     DFB_REQUIRE(workspace_doubles >= need, "workspace of %lld doubles is smaller than the %lld dfb_track_workspace_doubles asks for",
                 (long long)workspace_doubles, (long long)need);
-    TrackParams P;
-    for (int i = 0; i < 9; ++i) P.Kinv[i] = Kinv[i];
-    for (int i = 0; i < 12; ++i) P.lw[i] = lw34[i];
-    for (int i = 0; i < 3; ++i) P.center[i] = center[i];
-    P.scale = scale; P.half = tsdf_res / 2.0; P.tdist = tdist; P.delta = delta;
-    P.rows = rows; P.cols = cols; P.stride = stride;
-    P.rows_s = (rows + stride - 1) / stride; P.cols_s = (cols + stride - 1) / stride;
-    P.rx = vol->rx; P.ry = vol->ry; P.rz = vol->rz;
     const cudaStream_t s = (cudaStream_t)stream;
     const int64_t blocks = track_blocks(rows, cols, stride);
     track_pixel_kernel<<<(unsigned)blocks, TRACK_THREADS, 0, s>>>(P, vol->tsdf, vol->weight, depth, workspace, residual);

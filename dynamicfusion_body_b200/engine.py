@@ -294,30 +294,36 @@ def fill_lw(s, lw):
             s.lw[i] = float(lw[i])
 
 
-def make_views(depths, K, Kinv=None, extrinsics=None):
-    """depths: CUDA float32 tensor (V,rows,cols) (negative depth, 0 = no data)."""
-    if depths.dim() == 2:
-        depths = depths[None]
-    assert depths.is_cuda and depths.dtype == torch.float32 and depths.is_contiguous()
+def views_struct(n_views, rows, cols, K, Kinv=None, extrinsics=None, depth_ptrs=()):
+    """dfb_views of n_views cameras: intrinsics K and Kinv (the inverse of K when None), rows x cols images, the addresses of the
+    depth maps (none for cameras without depth maps) and, when given, one 3x4 world -> camera extrinsic per view."""
     K = np.asarray(K, dtype=np.float64)
     Kinv = np.linalg.inv(K) if Kinv is None else np.asarray(Kinv, dtype=np.float64)
     v = _capi.Views()
-    v.n_views = depths.shape[0]
-    if v.n_views > _capi.DFB_MAX_VIEWS:
-        raise ValueError("at most %d views per pass" % _capi.DFB_MAX_VIEWS)
-    for i in range(v.n_views):
-        v.depth[i] = depths[i].data_ptr()
-    v.rows, v.cols = int(depths.shape[1]), int(depths.shape[2])
+    v.n_views = n_views
+    for i, p in enumerate(depth_ptrs):
+        v.depth[i] = p
+    v.rows, v.cols = int(rows), int(cols)
     for i in range(9):
         v.K[i] = float(K.ravel()[i])
         v.Kinv[i] = float(Kinv.ravel()[i])
     v.has_extrinsics = 0 if extrinsics is None else 1
     if extrinsics is not None:
-        E = np.asarray(extrinsics, dtype=np.float64).reshape(v.n_views, 12)
-        for j in range(v.n_views):
+        E = np.asarray(extrinsics, dtype=np.float64).reshape(n_views, 12)
+        for j in range(n_views):
             for i in range(12):
                 v.E[j][i] = float(E[j, i])
     return v
+
+
+def make_views(depths, K, Kinv=None, extrinsics=None):
+    """depths: CUDA float32 tensor (V,rows,cols) (negative depth, 0 = no data)."""
+    if depths.dim() == 2:
+        depths = depths[None]
+    assert depths.is_cuda and depths.dtype == torch.float32 and depths.is_contiguous()
+    if depths.shape[0] > _capi.DFB_MAX_VIEWS:
+        raise ValueError("at most %d views per pass" % _capi.DFB_MAX_VIEWS)
+    return views_struct(depths.shape[0], depths.shape[1], depths.shape[2], K, Kinv, extrinsics, [d.data_ptr() for d in depths])
 
 
 def _mask_bufs(vol, want):
@@ -491,23 +497,10 @@ def corr_projective(warped_pts, warped_normals, views, max_distance, min_normal_
 def camera_views(K, rows, cols, extrinsics=None, n_views=None):
     """dfb_views of cameras without depth maps (the input of `render`): intrinsics K, image size, and either `n_views` copies of
     the camera (default 1) or one view per 3x4 extrinsic of `extrinsics` (world -> camera, as in `make_views`)."""
-    K = np.asarray(K, dtype=np.float64)
-    v = _capi.Views()
-    v.n_views = (1 if n_views is None else int(n_views)) if extrinsics is None else len(extrinsics)
-    if not 1 <= v.n_views <= _capi.DFB_MAX_VIEWS:
+    n = (1 if n_views is None else int(n_views)) if extrinsics is None else len(extrinsics)
+    if not 1 <= n <= _capi.DFB_MAX_VIEWS:
         raise ValueError("between 1 and %d views per pass" % _capi.DFB_MAX_VIEWS)
-    v.rows, v.cols = int(rows), int(cols)
-    Kinv = np.linalg.inv(K)
-    for i in range(9):
-        v.K[i] = float(K.ravel()[i])
-        v.Kinv[i] = float(Kinv.ravel()[i])
-    v.has_extrinsics = 0 if extrinsics is None else 1
-    if extrinsics is not None:
-        E = np.asarray(extrinsics, dtype=np.float64).reshape(v.n_views, 12)
-        for j in range(v.n_views):
-            for i in range(12):
-                v.E[j][i] = float(E[j, i])
-    return v
+    return views_struct(n, rows, cols, K, None, extrinsics)
 
 
 def render_workspace(n_faces, views, device=None):

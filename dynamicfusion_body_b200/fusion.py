@@ -505,11 +505,8 @@ class Fusion(_FusionBase):
             self._faces = None
             self._relink_nodes()
 
-    def _associate_projective(self, depths, extrinsics, max_distance, min_normal_dot, prune_result):
-        if self._vertices is None or self._normals is None:
-            raise ValueError('canonical vertices/normals have not been set')
-        if self._K is None:
-            raise ValueError('camera intrinsics K have not been set')
+    def _depth_frames(self, depths, extrinsics):
+        """depths as a (views, rows, cols) float32 tensor on the device, with one extrinsic per view when they are given."""
         d = engine._to_dev(depths, torch.float32, self._device)
         if d.dim() == 2:
             d = d[None]
@@ -517,6 +514,14 @@ class Fusion(_FusionBase):
             raise ValueError('depth maps must be (rows, cols) or (views, rows, cols)')
         if extrinsics is not None and len(extrinsics) != d.shape[0]:
             raise ValueError('length of camera matrix array must equal that of depth maps')
+        return d
+
+    def _associate_projective(self, depths, extrinsics, max_distance, min_normal_dot, prune_result):
+        if self._vertices is None or self._normals is None:
+            raise ValueError('canonical vertices/normals have not been set')
+        if self._K is None:
+            raise ValueError('camera intrinsics K have not been set')
+        d = self._depth_frames(depths, extrinsics)
         md = self._tdist if max_distance is None else float(max_distance)
         views = engine.make_views(d, self._K, self._Kinv, extrinsics)
         loc = self._dev(self._neighbor_look_up, torch.int32).reshape(len(self._vertices), -1)
@@ -574,13 +579,7 @@ class Fusion(_FusionBase):
             self._Kinv = np.linalg.inv(self._K)
         if self._K is None:
             raise ValueError('camera intrinsics K have not been set')
-        d = engine._to_dev(depths, torch.float32, self._device)
-        if d.dim() == 2:
-            d = d[None]
-        if d.dim() != 3:
-            raise ValueError('depth maps must be (rows, cols) or (views, rows, cols)')
-        if extrinsics is not None and len(extrinsics) != d.shape[0]:
-            raise ValueError('length of camera matrix array must equal that of depth maps')
+        d = self._depth_frames(depths, extrinsics)
         return engine.update_projective(self._vol, self._wf, self._lw, d, self._K, self._Kinv, extrinsics, self._tdist, wmax,
                                         mode=self._mode if mode is None else mode, want_masks=want_masks)
 

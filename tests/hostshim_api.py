@@ -1,25 +1,27 @@
-"""TEST INFRASTRUCTURE: numpy-facing wrapper of tests/hostshim/libdfb_hostshim.so -- the host build of the
-kernels' per-voxel logic (see tests/hostshim/hostshim.cpp).  Lets the CPU suite check the two arithmetic
-tiers against the oracle without a GPU."""
+"""TEST INFRASTRUCTURE: numpy-facing wrapper of tests/hostshim/libdfb_hostshim.so -- the host build of the kernels' per-element
+logic and of the entry points' own argument checks and parameter set-up (see tests/hostshim/*.cpp).  Lets the CPU suite check the
+arithmetic against the oracle without a GPU."""
 import ctypes as C
+import glob
 import os
 import subprocess
 
 import numpy as np
 
-from dynamicfusion_body_b200 import _capi
+from dynamicfusion_body_b200 import _capi, engine
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
-_SRC = os.path.join(_HERE, "hostshim", "hostshim.cpp")
 _SO = os.path.join(_HERE, "hostshim", "libdfb_hostshim.so")
-_CSRC = os.path.join(os.path.dirname(_HERE), "dynamicfusion_body_b200", "csrc")
+_ROOT = os.path.dirname(_HERE)
 
 
 def build(force=False):
-    deps = [_SRC] + [os.path.join(_CSRC, f) for f in ("dfb_math.h", "dfb_voxel.h", "dfb_params.h", "dfb_gn.h", "dfb_brick.h", "dfb_mc.h", "dfb_mc_table.h")]
+    srcs = sorted(glob.glob(os.path.join(_HERE, "hostshim", "*.cpp")))
+    deps = [f for f in glob.glob(os.path.join(_HERE, "hostshim", "*")) if not f.endswith(".so")]
+    deps += glob.glob(os.path.join(_ROOT, "dynamicfusion_body_b200", "csrc", "*.h")) + [os.path.join(_ROOT, "include", "dfb.h")]
     if not force and os.path.isfile(_SO) and all(os.path.getmtime(_SO) >= os.path.getmtime(d) for d in deps):
         return _SO
-    subprocess.check_call(["g++", "-O2", "-std=c++17", "-ffp-contract=off", "-fPIC", "-shared", _SRC, "-o", _SO])
+    subprocess.check_call(["g++", "-O2", "-std=c++17", "-ffp-contract=off", "-fPIC", "-shared"] + srcs + ["-o", _SO])
     return _SO
 
 
@@ -30,7 +32,7 @@ def lib():
     global _lib
     if _lib is None:
         _lib = C.CDLL(build())
-        vp = C.c_void_p
+        vp, i, d = C.c_void_p, C.c_int, C.c_double
         _lib.hs_last_error.restype = C.c_char_p
         _lib.hs_nodes_pack.argtypes = [vp, vp, vp, C.c_int, vp]
         _lib.hs_tsdf_update_projective.argtypes = [C.POINTER(_capi.Volume), C.POINTER(_capi.WarpField), C.POINTER(_capi.Views),
@@ -40,6 +42,10 @@ def lib():
         _lib.hs_tsdf_update_volume.argtypes = [C.POINTER(_capi.Volume), C.POINTER(_capi.WarpField), vp, C.c_int, C.c_int, C.c_int,
                                                C.c_double, C.c_double, C.c_int, C.POINTER(_capi.Workspace), vp, vp]
         _lib.hs_warp_points.argtypes = [vp, vp, C.c_int64, vp, C.POINTER(_capi.WarpField), vp, vp]
+        _lib.hs_corr_projective.argtypes = [vp, vp, C.c_int64, C.POINTER(_capi.Views), d, d, vp, vp, vp]
+        _lib.hs_render.argtypes = [vp, C.c_int64, vp, C.c_int64, C.POINTER(_capi.Views), vp, vp, vp]
+        _lib.hs_track_normal_eq.argtypes = [C.POINTER(_capi.Volume), i, d, vp, vp, i, i, vp, vp, vp, i, d, d, vp, vp, vp]
+        _lib.hs_raycast.argtypes = [C.POINTER(_capi.Volume), i, d, vp, C.POINTER(_capi.Views), d, d, d, d, vp, vp]
     return _lib
 
 
@@ -137,28 +143,17 @@ def _ws():
     return w, counters
 
 
-def make_views(depths, K, Kinv, extrinsics=None):
+def _views(depths, K, Kinv, extrinsics=None):
+    """engine.views_struct over host depth maps; returns it with the arrays it points into."""
     depths = [np.ascontiguousarray(d, dtype=np.float32) for d in depths]
-    v = _capi.Views()
-    v.n_views = len(depths)
-    for i, d in enumerate(depths):
-        v.depth[i] = d.ctypes.data
-    v.rows, v.cols = depths[0].shape
-    for i in range(9):
-        v.K[i] = float(np.asarray(K).ravel()[i])
-        v.Kinv[i] = float(np.asarray(Kinv).ravel()[i])
-    v.has_extrinsics = 0 if extrinsics is None else 1
-    if extrinsics is not None:
-        for j in range(len(depths)):
-            for i in range(12):
-                v.E[j][i] = float(np.asarray(extrinsics[j]).ravel()[i])
-    return v, depths
+    rows, cols = depths[0].shape
+    return engine.views_struct(len(depths), rows, cols, K, Kinv, extrinsics, [d.ctypes.data for d in depths]), depths
 
 
 def update_projective(tsdf, w, res, wf, depths, K, Kinv, tdist, extrinsics=None, wmax=100.0, mode=0, x0=0, x1=None):
     """tsdf, w: float32 slab arrays (modified in place). Returns (mask, frustum, cls, n_uncertain)."""
     x1 = res[0] if x1 is None else x1
-    views, keep = make_views(depths, K, Kinv, extrinsics)
+    views, keep = _views(depths, K, Kinv, extrinsics)
     ws, counters = _ws()
     n = tsdf.size
     mask = np.zeros(n, np.uint8); frus = np.zeros(n, np.uint8); cls = np.zeros(n, np.uint8)
@@ -204,6 +199,72 @@ def warp_points(pts, normals, idx, wf):
     s = wf.struct()
     _check(lib().hs_warp_points(_p(pts), _p(normals), len(pts), _p(idx), C.byref(s), _p(out), _p(outn)))
     return (out, outn) if normals is not None else out
+
+
+def corr_projective(warped_pts, warped_normals, depths, K, Kinv, max_distance, min_normal_dot, extrinsics=None):
+    """Host run of dfb_corr_projective: (view (m,) int32, cost (m,) float64, corr (m,3) float64)."""
+    wp = np.ascontiguousarray(warped_pts, dtype=np.float64).reshape(-1, 3)
+    wn = np.ascontiguousarray(warped_normals, dtype=np.float64).reshape(-1, 3)
+    views, keep = _views(depths, K, Kinv, extrinsics)
+    m = len(wp)
+    view = np.zeros(m, np.int32)
+    cost = np.zeros(m)
+    corr = np.zeros((m, 3))
+    _check(lib().hs_corr_projective(_p(wp), _p(wn), m, C.byref(views), float(max_distance), float(min_normal_dot), _p(view), _p(cost),
+                                    _p(corr)))
+    return view, cost, corr
+
+
+def render(pts, faces, K, rows, cols, extrinsics=None, n_views=None):
+    """Host run of dfb_render: (depth (V,rows,cols) float32, face (V,rows,cols) int32, normal (V,rows,cols,3) float32)."""
+    P = np.ascontiguousarray(pts, dtype=np.float64).reshape(-1, 3)
+    F = np.ascontiguousarray(faces, dtype=np.int32).reshape(-1, 3)
+    views = engine.camera_views(K, rows, cols, extrinsics, n_views)
+    V = views.n_views
+    depth = np.zeros((V, rows, cols), np.float32)
+    face = np.zeros((V, rows, cols), np.int32)
+    normal = np.zeros((V, rows, cols, 3), np.float32)
+    _check(lib().hs_render(_p(P), len(P), _p(F), len(F), C.byref(views), _p(depth), _p(face), _p(normal)))
+    return depth, face, normal
+
+
+def normal_eq(tsdf, weight, tsdf_res, scale, center, depth, Kinv, lw34, stride, tdist, delta):
+    """Host run of dfb_track_normal_eq: (sums (29,), residual (rows_s, cols_s) NaN = none, jac (rows_s, cols_s, 6) 0 = none)."""
+    T = np.ascontiguousarray(tsdf, dtype=np.float32)
+    W = np.ascontiguousarray(weight, dtype=np.float32)
+    dm = np.ascontiguousarray(depth, dtype=np.float32)
+    rows, cols = dm.shape
+    rs, cs = (rows + stride - 1) // stride, (cols + stride - 1) // stride
+    ctr = np.ascontiguousarray(center, dtype=np.float64).reshape(3)
+    Ki = np.ascontiguousarray(Kinv, dtype=np.float64).reshape(3, 3)
+    K = np.linalg.inv(Ki)
+    lw = np.ascontiguousarray(lw34, dtype=np.float64).reshape(12)
+    out = np.zeros(29)
+    res = np.zeros((rs, cs))
+    jac = np.zeros((rs, cs, 6))
+    vol = _vol(T, W, T.shape, 0, T.shape[0])
+    _check(lib().hs_track_normal_eq(C.byref(vol), int(tsdf_res), float(scale), _p(ctr), _p(dm), rows, cols, _p(K), _p(Ki), _p(lw),
+                                    int(stride), float(tdist), float(delta), _p(out), _p(res), _p(jac)))
+    return out, res, jac
+
+
+def raycast(tsdf, weight, tsdf_res, scale, center, tdist, K, rows, cols, extrinsics=None, step=None, z_near=0.0, z_far=None):
+    """Host run of dfb_raycast with the arguments of oracle/raycast.py:raycast (views from engine.camera_views; z_far defaults to
+    engine.raycast_far as in engine.raycast): (depth (V,rows,cols) float32, normal (V,rows,cols,3) float32)."""
+    T = np.ascontiguousarray(tsdf, dtype=np.float32)
+    W = np.ascontiguousarray(weight, dtype=np.float32)
+    views = engine.camera_views(K, rows, cols, extrinsics)
+    ctr = np.ascontiguousarray(center, dtype=np.float64).reshape(3)
+    step = float(scale) if step is None else float(step)
+    if z_far is None:
+        z_far = max(engine.raycast_far(T.shape, tsdf_res, views, scale, ctr), z_near + step)
+    V = views.n_views
+    depth = np.zeros((V, rows, cols), np.float32)
+    normal = np.zeros((V, rows, cols, 3), np.float32)
+    vol = _vol(T, W, T.shape, 0, T.shape[0])
+    _check(lib().hs_raycast(C.byref(vol), int(tsdf_res), float(scale), _p(ctr), C.byref(views), float(tdist), step, float(z_near),
+                            float(z_far), _p(depth), _p(normal)))
+    return depth, normal
 
 
 # ---- Gauss-Newton path ------------------------------------------------------------------------------------------

@@ -6,7 +6,6 @@ import ctypes
 import numpy as np
 import pytest
 
-import assoc_shim
 import hostshim_api as hs
 from dynamicfusion_body_b200 import synth
 from oracle import assoc as oa
@@ -38,7 +37,7 @@ def _both(pts, nrm, dms, md=MD, mnd=0.5, extrinsics=None):
     pts = np.atleast_2d(np.asarray(pts, np.float64))
     nrm = np.atleast_2d(np.asarray(nrm, np.float64))
     dms = np.asarray(dms, np.float32).reshape(-1, ROWS, COLS) if np.ndim(dms) == 2 else np.asarray(dms, np.float32)
-    hv, hc, hp = assoc_shim.corr_projective(pts, nrm, dms, K, KINV, md, mnd, extrinsics)
+    hv, hc, hp = hs.corr_projective(pts, nrm, dms, K, KINV, md, mnd, extrinsics)
     ov, oc, op = oa.associate(pts, nrm, dms, K, KINV, md, mnd, extrinsics)
     _assert_bits(hv, hc, hp, ov, oc, op)
     return ov, oc, op
@@ -146,7 +145,7 @@ def test_scene_host_equals_oracle(n_views, k):
     wf = hs.HostWarpField(sc.node_pos, sc.node_dq, np.float32(sc.node_w), sc.k, lw=sc.lw)
     # the body-mesh fixture's normals point into the body; association wants them pointing out (as marching cubes of a TSDF)
     wv, wn = hs.warp_points(sc.vertices, -sc.normals, sc.vert_knn, wf)
-    hv, hc, hp = assoc_shim.corr_projective(wv, wn, sc.depths, sc.K, sc.Kinv, sc.tdist, 0.5, sc.extrinsics)
+    hv, hc, hp = hs.corr_projective(wv, wn, sc.depths, sc.K, sc.Kinv, sc.tdist, 0.5, sc.extrinsics)
     ov, oc, op = oa.associate(wv, wn, sc.depths, sc.K, sc.Kinv, sc.tdist, 0.5, sc.extrinsics)
     _assert_bits(hv, hc, hp, ov, oc, op)
     frac = float((ov >= 0).mean())

@@ -8,7 +8,7 @@ import ctypes
 import numpy as np
 import pytest
 
-import raycast_shim
+import hostshim_api as hs
 from dynamicfusion_body_b200 import engine, synth
 from oracle import raycast as orc
 from oracle import track as otr
@@ -27,7 +27,7 @@ def _both(T, W, res, scale, center, tdist, Kc, rows, cols, E, step=None, z_near=
     step = float(scale) if step is None else float(step)
     if z_far is None:
         z_far = max(engine.raycast_far(np.shape(T), res, engine.camera_views(Kc, rows, cols, E), scale, center), z_near + step)
-    dh, nh = raycast_shim.raycast(T, W, res, scale, center, tdist, Kc, rows, cols, E, step, z_near, z_far)
+    dh, nh = hs.raycast(T, W, res, scale, center, tdist, Kc, rows, cols, E, step, z_near, z_far)
     out = [orc.raycast_view(T, W, res, scale, center, tdist, np.linalg.inv(Kc), e, rows, cols, step, z_near, z_far) for e in E]
     do, no, zo = (np.stack([o[i] for o in out]) for i in range(3))
     assert np.array_equal(dh.view(np.uint32), do.view(np.uint32))

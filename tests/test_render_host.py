@@ -7,7 +7,7 @@ import ctypes
 import numpy as np
 import pytest
 
-import render_shim
+import hostshim_api as hs
 from dynamicfusion_body_b200 import synth
 from oracle import render as orr
 
@@ -32,7 +32,7 @@ def _both(pts, faces, extrinsics=None, rows=ROWS, cols=COLS, k=K):
     """host build and oracle on the same input; asserts they agree bit for bit and returns the oracle's view 0 (or all views)."""
     pts = np.asarray(pts, np.float64).reshape(-1, 3)
     faces = np.asarray(faces, np.int32).reshape(-1, 3)
-    h = render_shim.render(pts, faces, k, rows, cols, extrinsics)
+    h = hs.render(pts, faces, k, rows, cols, extrinsics)
     o = orr.render(pts, faces, k, rows, cols, extrinsics)
     _assert_bits(h, o)
     return tuple(a[0] for a in o) if extrinsics is None else o

@@ -7,7 +7,7 @@ import ctypes
 import numpy as np
 import pytest
 
-import track_shim
+import hostshim_api as hs
 from dynamicfusion_body_b200 import engine, synth
 from oracle import track as otr
 from track_scenes import Ring, perturb, pose_error
@@ -23,7 +23,7 @@ IDENT = np.concatenate([np.eye(3), np.zeros((3, 1))], 1)
 def _both(T, W, res, scale, center, dm, Kinv, lw, stride, tdist, delta):
     """host build and oracle on the same input: residual maps and Jacobians bit for bit, sums to rounding; returns the oracle's
     per-pixel dict and sums."""
-    sh, rh, jh = track_shim.normal_eq(T, W, res, scale, center, dm, Kinv, lw, stride, tdist, delta)
+    sh, rh, jh = hs.normal_eq(T, W, res, scale, center, dm, Kinv, lw, stride, tdist, delta)
     so, ro = otr.normal_eq(T, W, res, scale, center, dm, Kinv, lw, stride, tdist, delta, want_residual=True)
     px = otr.pixels(T, W, res, scale, center, dm, Kinv, lw, stride, tdist)
     assert np.array_equal(rh.view(np.uint64), ro.view(np.uint64))
@@ -152,7 +152,7 @@ def test_pose_looking_away_contributes_nothing(ring64):
     eye = -lw0[:, :3].T @ lw0[:, 3]
     away = synth.look_at_extrinsic(eye, 2 * eye - rg.target)            # the same camera turned to face away from the body
     sums = otr.normal_eq(T, W, rg.res, rg.scale, rg.center, dm, rg.Kinv, away, 1, rg.tdist, 0.5 * rg.tdist)
-    sh, _, _ = track_shim.normal_eq(T, W, rg.res, rg.scale, rg.center, dm, rg.Kinv, away, 1, rg.tdist, 0.5 * rg.tdist)
+    sh, _, _ = hs.normal_eq(T, W, rg.res, rg.scale, rg.center, dm, rg.Kinv, away, 1, rg.tdist, 0.5 * rg.tdist)
     assert sums[28] == 0 and np.all(sh == 0)
     with pytest.raises(ValueError, match="pixels"):
         engine.track_rigid(lambda lw, s: otr.normal_eq(T, W, rg.res, rg.scale, rg.center, dm, rg.Kinv, lw, s, rg.tdist, 0.5 * rg.tdist), away)
